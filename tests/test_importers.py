@@ -211,14 +211,11 @@ def test_hdr_round_trip(host, tmp_path):
     assert np.abs(y - x).max() <= x.max(axis=2, keepdims=True).max() / 128  # 8-bit mantissa shared exponent
 
 
-REF_HDR = "/root/reference/data/abandoned_tank_farm_04_1k.hdr"
-
-
-@pytest.mark.skipif(not os.path.exists(REF_HDR), reason="the reference's environment map only exists in the build container")
 def test_hdr_decoder_on_the_reference_map_matches_opencv(host):
+    """The reference's own environment map (data/abandoned_tank_farm_04_1k.hdr), committed as tests/golden's fixture."""
     cv2 = pytest.importorskip("cv2")
-    img = host.load_hdr(REF_HDR)
-    ref = cv2.imread(REF_HDR, cv2.IMREAD_UNCHANGED)[..., ::-1]
+    img = host.load_hdr(host.TANK_FARM_HDR)
+    ref = cv2.imread(host.TANK_FARM_HDR, cv2.IMREAD_UNCHANGED)[..., ::-1]
     assert img.shape == (512, 1024, 3) and np.array_equal(img, ref)
 
 

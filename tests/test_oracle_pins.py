@@ -3,13 +3,15 @@
 The reference holds no golden vectors for the rendering path (SURVEY.md §4: 7 unit tests, none on the
 path's arithmetic) and cannot be compiled here, so parity is formally UNPINNED.  What can be pinned:
   * the Sobol tables: re-derived from the Joe-Kuo direction numbers (scipy's copy) and bit-identical to
-    the reference's sobolmatrices.rs when that checkout is present
+    the reference's sobolmatrices.rs (digests of its tables under tests/golden/)
   * the Sobol sequence itself against scipy.stats.qmc.Sobol (independent implementation)
   * the helper known-answer tests the reference does have (src/common/math.rs:264-299)
   * documented quirks (next_float_down, pixel-corner clamping), analytic properties of the lobes
   * committed golden vectors of the oracle (tests/golden/) so that any later drift is caught
 """
 import ctypes as C
+import hashlib
+import json
 import os
 import re
 import struct
@@ -50,9 +52,15 @@ def test_sobol_tables_rederive_from_joe_kuo():
     assert all(list(a) == b for a, b in zip(vdc, dv)) and all(list(a) == b for a, b in zip(vdc_inv, di))
     assert mats.shape == (1024, 52) and len(vdc) == 25 and len(vdc_inv) == 26
     assert [len(v) for v in vdc] == [52 - 2 * m for m in range(1, 26)] and [len(v) for v in vdc_inv] == [2 * m for m in range(1, 27)]
-    if os.path.exists(g.REF):  # the reference's own tables (src/pathtracer/sobolmatrices.rs:5-7, 53463, 54155)
-        rm, rv, ri = g.parse_reference()
-        assert np.array_equal(rm, mats) and rv == dv and ri == di
+    # the reference's own tables (src/pathtracer/sobolmatrices.rs:5-7, 53463, 54155), stored as digests
+    with open(os.path.join(ROOT, "tests", "golden", "sobol_reference_tables.json")) as f:
+        ref = json.load(f)
+
+    def digest(tables):
+        return hashlib.sha256(b"".join(np.asarray(t, dtype="<u8").tobytes() for t in tables)).hexdigest()
+
+    assert hashlib.sha256(dm.astype("<u4").tobytes()).hexdigest() == ref["SOBOL_MATRICES_32"]
+    assert digest(dv) == ref["VD_C_SOBOL_MATRICES"] and digest(di) == ref["VD_C_SOBOL_MATRICES_INV"]
 
 
 def test_sobol_sample_matches_scipy_sequence(oracle):
@@ -369,16 +377,31 @@ def test_product_package_does_not_import_the_oracle():
                 assert "oracle" not in txt.lower(), os.path.join(dirpath, f)
 
 
+_NO_DEVICE_CHILD = """
+import ctypes as C
+import sys
+
+import pytest
+
+sys.path.insert(0, sys.argv[1])
+import pathtracer_rs_b200.gpu as gpu
+
+n = C.c_int32(-1)
+rc = gpu.lib().ptrs_device_count(C.byref(n))
+assert rc != 0 or n.value == 0, n.value
+flat = None
+with pytest.raises((gpu.PtrsError, RuntimeError)):
+    import pathtracer_rs_b200.host as host
+
+    flat, _ = host.make_scene(host.SCENE_CORNELL, res=(8, 8))
+    gpu.RenderScene(flat)
+"""
+
+
 def test_no_cpu_fallback_without_a_device():
-    import pathtracer_rs_b200.gpu as gpu
+    """In a child process that sees no CUDA device (on a GPU machine as well), the render path raises."""
+    import subprocess
 
-    n = C.c_int32(-1)
-    rc = gpu.lib().ptrs_device_count(C.byref(n))
-    if rc == 0 and n.value > 0:
-        pytest.skip("a CUDA device is present")
-    flat = None
-    with pytest.raises((gpu.PtrsError, RuntimeError)):
-        import pathtracer_rs_b200.host as host
-
-        flat, _ = host.make_scene(host.SCENE_CORNELL, res=(8, 8))
-        gpu.RenderScene(flat)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHILD, ROOT], env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
