@@ -982,6 +982,189 @@ PT_DEV void trace_counted(const DevScene& sc, uint32_t n_items, uint32_t* ticket
   }
 }
 
+// ---- any-hit walk over the occlusion tree ----------------------------------------------------------------
+// An any-hit ray keeps its t_max until the first hit ends it, so the reference's walk (accelerator.rs:431-475) tests a
+// triangle exactly when the slab test of every box on the way to its leaf passes, in whatever order.  Every interior box of
+// the reference-built tree contains its children's boxes (ptrs_scene_create checks it before it builds this tree), and
+// with nested boxes the slab test of the inner box passing implies that of the outer one (float subtraction and
+// multiplication are monotonic; tests/test_occlusion_tree.py sweeps the NaN / infinity / signed-zero cases of box_geom).
+// So a triangle is tested iff its own leaf's box passes, and any tree whose child slots hold reference boxes, with the
+// reference's leaves under their own boxes, gives the reference's occlusion answer bit for bit in any visit order.
+//
+// The occlusion tree is that: every 128-byte wide node holds up to four reference nodes (a node and the interior
+// descendants the collapse replaced are skipped: their boxes contain the ones tested below them).  Layout, by plane:
+//   float4 [0..6)  min.x, max.x, min.y, max.y, min.z, max.z of the four slots
+//   float4 [6]     four child words: bit 31 clear = wide node index; set = leaf, (n_prims - 1) << 27 | first primitive;
+//                  PT_W_NONE = empty slot (its box is empty, and the word is checked as well)
+//   float4 [7]     unused
+// Stack entries are child words: 4 bytes, no entry distance (nothing is re-tested at pop time, t_max does not change).
+#define PT_W_NONE 0xffffffffu
+#define PT_W_LEAF_BIT 0x80000000u
+#define PT_W_IS_LEAF(w) (((w) & PT_W_LEAF_BIT) != 0u && (w) != PT_W_NONE)
+#define PT_W_IS_INTERIOR(w) (((w) & PT_W_LEAF_BIT) == 0u)
+#define PT_W_LEAF_OFF(w) ((w) & 0x07ffffffu)
+#define PT_W_LEAF_CNT(w) ((((w) >> 27) & 15u) + 1u)
+// up to three entries per wide level (a node's fourth entered child is the next node in hand); the wide tree is no deeper
+// than the reference's, which ptrs_scene_create limits to 64 levels
+#define PT_OSTACK_SIZE (3 * PT_STACK_SIZE)
+
+// Warp refill, box phase with one parked leaf, triangle phase: trace_fast's scheme without ordering obligations.
+// Work as for trace_fast; every ray is traced as an any-hit ray.
+template <class Work>
+PT_DEV void trace_occlusion(const DevScene& sc, uint32_t n_items, uint32_t* ticket, Work& work) {
+  if (sc.n_wnodes == 0) {
+    trace_empty(n_items, ticket, work);
+    return;
+  }
+  const uint32_t FULL = 0xffffffffu;
+  const int box_min = (int)sc.box_min;
+  uint32_t stack[PT_OSTACK_SIZE];
+  int sp_ = 0;
+  uint32_t cur = PT_W_NONE;         // entry in hand: wide node, leaf, or none
+  uint32_t pl_off = 0, pl_cnt = 0;  // parked leaf: next primitive, triangles left (0 = none)
+  uint32_t rbits = 0;               // PT_RB_LIVE, kz
+  bool exhausted = n_items == 0;
+  uint32_t item = 0;
+  V3 o = mk3(0, 0, 0), inv_dir = mk3(0, 0, 0);
+  float sx = 0.f, sy = 0.f, sz = 0.f;
+  float t_max = 0.f;
+  int hit_prim = -1;
+
+  auto start_ray = [&](const LaneRay& r) {
+    o = r.o;
+    inv_dir = mk3(1.0f / r.d.x, 1.0f / r.d.y, 1.0f / r.d.z);
+    const RayPre rp = ray_precompute(r.d);
+    sx = rp.sx;
+    sy = rp.sy;
+    sz = rp.sz;
+    rbits = PT_RB_LIVE | ((uint32_t)rp.kz << PT_RB_KZ_SHIFT);
+    t_max = r.t_max;
+    hit_prim = -1;
+    sp_ = 0;
+    pl_cnt = 0;
+    cur = 0u;  // the root's own box is not tested: it contains every leaf box
+  };
+
+  for (;;) {
+    // ---- refill ------------------------------------------------------------------------------------
+    const uint32_t idle = __ballot_sync(FULL, !(rbits & PT_RB_LIVE));
+    if (!exhausted && (__popc(idle) >= PT_REFILL_IDLE)) {
+      const int lane = threadIdx.x & 31;
+      const int leader = __ffs(idle) - 1;
+      uint32_t base = 0;
+      if (lane == leader) base = atomicAdd(ticket, (uint32_t)__popc(idle));
+      base = __shfl_sync(FULL, base, leader);
+      if (base + (uint32_t)__popc(idle) >= n_items) exhausted = true;
+      if (!(rbits & PT_RB_LIVE)) {
+        const uint32_t i = base + (uint32_t)__popc(idle & ((1u << lane) - 1u));
+        if (i < n_items) {
+          LaneRay r;
+          if (work.begin(i, &r)) {
+            item = i;
+            start_ray(r);
+          }
+        }
+      }
+    }
+    if (__ballot_sync(FULL, rbits & PT_RB_LIVE) == 0) {
+      if (exhausted) break;
+      continue;
+    }
+
+    // ---- box phase ------------------------------------------------------------------------------------
+    // (a lane without a ray has no entry in hand, an empty stack and no parked leaf)
+    auto box_step = [&]() {
+      if (cur == PT_W_NONE && sp_ > 0) cur = stack[--sp_];
+      if (PT_W_IS_LEAF(cur) && pl_cnt == 0u) {
+        pl_off = PT_W_LEAF_OFF(cur);
+        pl_cnt = PT_W_LEAF_CNT(cur);
+        cur = PT_W_NONE;
+      }
+      if (!PT_W_IS_INTERIOR(cur)) return;
+      const float4* nd = sc.wnodes + 8 * (size_t)cur;
+      const float4 lx = __ldg(nd), hx = __ldg(nd + 1), ly = __ldg(nd + 2), hy = __ldg(nd + 3), lz = __ldg(nd + 4), hz = __ldg(nd + 5);
+      const uint4 ch = __ldg(reinterpret_cast<const uint4*>(nd + 6));
+      const bool nx = inv_dir.x < 0.0f, ny = inv_dir.y < 0.0f, nz = inv_dir.z < 0.0f;
+      cur = PT_W_NONE;
+      auto child = [&](float x0, float x1, float y0, float y1, float z0, float z1, uint32_t w) {
+        NodeLoad n;
+        n.a = make_float4(x0, y0, z0, x1);
+        n.b = make_float4(y1, z1, 0.f, 0.f);
+        float te;
+        if (box_geom(n, o, inv_dir, nx, ny, nz, &te) && te < t_max && w != PT_W_NONE) {
+          if (PT_W_IS_LEAF(w) && pl_cnt == 0u) {
+            pl_off = PT_W_LEAF_OFF(w);
+            pl_cnt = PT_W_LEAF_CNT(w);
+          } else if (cur == PT_W_NONE) {
+            cur = w;
+          } else if (sp_ < PT_OSTACK_SIZE) {  // always true, see PT_OSTACK_SIZE
+            stack[sp_++] = w;
+          }
+        }
+      };
+      child(lx.x, hx.x, ly.x, hy.x, lz.x, hz.x, ch.x);
+      child(lx.y, hx.y, ly.y, hy.y, lz.y, hz.y, ch.y);
+      child(lx.z, hx.z, ly.z, hy.z, lz.z, hz.z, ch.z);
+      child(lx.w, hx.w, ly.w, hy.w, lz.w, hz.w, ch.w);
+    };
+    for (;;) {
+      const bool live = (rbits & PT_RB_LIVE) != 0;
+      const bool can_box = PT_W_IS_INTERIOR(cur) || (cur == PT_W_NONE && sp_ > 0) || (PT_W_IS_LEAF(cur) && pl_cnt == 0u);
+      const uint32_t bmask = __ballot_sync(FULL, can_box);
+      if (bmask == 0) break;
+      if (__popc(bmask) < box_min && __ballot_sync(FULL, live && !can_box) != 0) break;
+#pragma unroll
+      for (int rep = 0; rep < PT_BOX_STEPS; ++rep) box_step();
+    }
+
+    // ---- triangle phase: the parked leaf, then the leaf in hand ---------------------------------------
+    auto tri_step = [&]() {
+      if (pl_cnt == 0u && PT_W_IS_LEAF(cur)) {
+        pl_off = PT_W_LEAF_OFF(cur);
+        pl_cnt = PT_W_LEAF_CNT(cur);
+        cur = PT_W_NONE;
+      }
+      if (pl_cnt != 0u) {
+        const uint32_t prim = pl_off;
+        const float4 v0 = __ldg(sc.tri_verts + 3 * (size_t)prim);
+        const float4 v1 = __ldg(sc.tri_verts + 3 * (size_t)prim + 1);
+        const float4 v2 = __ldg(sc.tri_verts + 3 * (size_t)prim + 2);
+        ++pl_off;
+        --pl_cnt;
+        RayPre rp;
+        rp.kz = (int)((rbits >> PT_RB_KZ_SHIFT) & 3u);
+        rp.sx = sx;
+        rp.sy = sy;
+        rp.sz = sz;
+        float t, b0, b1, b2;
+        if (tri_core(mk3(v0), mk3(v1), mk3(v2), o, rp, t_max, &t, &b0, &b1, &b2) &&
+            !tri_post_reject(sc, (int)prim, mk3(v0), mk3(v1), mk3(v2), __float_as_uint(v2.w), b0, b1, b2, false)) {
+          hit_prim = (int)prim;  // intersect_p returns at the first hit (accelerator.rs:435-442)
+          pl_cnt = 0;
+          sp_ = 0;
+          cur = PT_W_NONE;
+        }
+      }
+    };
+    for (;;) {
+      const bool has = pl_cnt != 0u || PT_W_IS_LEAF(cur);
+      if (__ballot_sync(FULL, has) == 0) break;
+      tri_step();
+    }
+
+    // ---- rays that ran out of nodes --------------------------------------------------------------------
+    if ((rbits & PT_RB_LIVE) && cur == PT_W_NONE && sp_ == 0 && pl_cnt == 0u) {
+      DevHit h;
+      h.prim = hit_prim;
+      h.t = t_max;
+      h.b0 = h.b1 = h.b2 = 0.f;
+      LaneRay r;
+      if (work.end(item, h, hit_prim >= 0, &r)) start_ray(r);
+      else rbits = 0;
+    }
+  }
+}
+
 template <bool COUNT, bool DIST, class Work>
 PT_DEV void trace_stream(const DevScene& sc, uint32_t n_items, uint32_t* ticket, Work& work, uint32_t* c_nodes, uint32_t* c_tris) {
   if (COUNT) trace_counted(sc, n_items, ticket, work, c_nodes, c_tris);  // (reads sc.dist_order at run time)

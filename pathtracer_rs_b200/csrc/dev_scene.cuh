@@ -58,6 +58,10 @@ struct DevScene {
   // differentials (MIPMap::lookup's filter width, texture.rs:431-445).  Without one, shade skips
   // compute_differentials — every value it would produce is unread.
   uint32_t uses_differentials;
+  // occlusion tree (any-hit rays only, trace_occlusion): 128-byte wide nodes collapsed from the reference-built tree, 8
+  // float4 per node; n_wnodes == 0 when the scene has none (device-built tree, or a tree the collapse does not accept)
+  const float4* wnodes;
+  uint32_t n_wnodes;
 };
 
 // tri_verts[3 * prim + 2].w packs: bits 0..7 mesh flags, bit 8 has-alpha, bits 9.. alpha texture id

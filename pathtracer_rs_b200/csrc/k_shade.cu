@@ -246,8 +246,12 @@ __global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_ker
     {
       const uint32_t nfl = push_nee ? __float_as_uint(nee.n3.w) : 0u;
       const uint32_t ma = __ballot_sync(0xffffffffu, push_nee), mb = __ballot_sync(0xffffffffu, push_ext);
-      const uint32_t ms = __ballot_sync(0xffffffffu, (nfl & PT_NEE_SHADOW) != 0), mm = __ballot_sync(0xffffffffu, (nfl & PT_NEE_MIS) != 0);
-      uint32_t ba = 0, bb = 0, br = 0;
+      // any-hit rays (shadow segments, MIS rays of infinite lights) fill q_ray from the bottom, closest-hit MIS rays (area
+      // lights) from the top down: connect traces the two lists with different kernels
+      const uint32_t ms = __ballot_sync(0xffffffffu, (nfl & PT_NEE_SHADOW) != 0);
+      const uint32_t mm = __ballot_sync(0xffffffffu, (nfl & (PT_NEE_MIS | PT_NEE_MIS_ANY)) == (PT_NEE_MIS | PT_NEE_MIS_ANY));
+      const uint32_t mc = __ballot_sync(0xffffffffu, (nfl & (PT_NEE_MIS | PT_NEE_MIS_ANY)) == PT_NEE_MIS);
+      uint32_t ba = 0, bb = 0, br = 0, bc = 0;
       if (lane == 0) {
         if (ma) {
           const unsigned long long both = atomicAdd(reinterpret_cast<unsigned long long*>(&ctr->n_nee),
@@ -255,11 +259,13 @@ __global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_ker
           ba = (uint32_t)both;
           br = (uint32_t)(both >> 32);
         }
+        if (mc) bc = atomicAdd(&ctr->n_ray_closest, (uint32_t)__popc(mc));
         if (mb) bb = atomicAdd(&ctr_next->n_ext, (uint32_t)__popc(mb));
       }
       ba = __shfl_sync(0xffffffffu, ba, 0);
       bb = __shfl_sync(0xffffffffu, bb, 0);
       br = __shfl_sync(0xffffffffu, br, 0);
+      bc = __shfl_sync(0xffffffffu, bc, 0);
       const uint32_t lt = (1u << lane) - 1u;
       if (push_nee) {
         const uint32_t k = ba + __popc(ma & lt);
@@ -269,7 +275,8 @@ __global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_ker
         st256(dst + 1, F8{nee.n2, nee.n3});
         st256(dst + 2, F8{nee.n4, nee.n5});
         if (nfl & PT_NEE_SHADOW) P.q_ray[br + __popc(ms & lt)] = 2u * k;
-        if (nfl & PT_NEE_MIS) P.q_ray[br + __popc(ms) + __popc(mm & lt)] = 2u * k + 1u;
+        if ((mm >> lane) & 1u) P.q_ray[br + __popc(ms) + __popc(mm & lt)] = 2u * k + 1u;
+        if ((mc >> lane) & 1u) P.q_ray[2u * rc.cap - 1u - (bc + __popc(mc & lt))] = 2u * k + 1u;
       }
       if (push_ext) q_ext_next[bb + __popc(mb & lt)] = p;
     }

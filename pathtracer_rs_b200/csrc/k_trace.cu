@@ -65,14 +65,17 @@ __global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) extend_kernel(const 
 // ---- connect ---------------------------------------------------------------------------------------
 // Rays of estimate_direct for the pending records: shade lists in q_ray the rays that exist, 2 * record for a
 // shadow segment (integrator.rs:66-78, light.rs:39-41, any-hit), 2 * record + 1 for a BSDF-sampled MIS ray
-// (integrator.rs:113-135, closest hit), so every work item is a ray and no lane idles on an absent one.  The kernel only traces: what was found goes to nee_res[i], and connect_resolve_kernel
+// (integrator.rs:113-135, closest hit), so every work item is a ray and no lane idles on an absent one.  Any-hit rays sit
+// at the bottom of q_ray (n_ray of them), closest-hit ones at the top (n_ray_closest): work item i < n_low is q_ray[i],
+// the rest count down from q_ray[2 * cap - 1].  The kernel only traces: what was found goes to nee_res[i], and connect_resolve_kernel
 // (k_misc.cu) evaluates emitted radiance and adds the bounce's direct lighting at full warp width.
 struct ConnectWork {
   const PathArrays& P;
+  uint32_t n_low, top;  // top = 2 * cap - 1
   uint32_t n_shadow, n_mis;
   uint32_t cur;  // 2 * record + kind of the ray in hand
   __device__ bool begin(uint32_t i, LaneRay* r) {
-    cur = P.q_ray[i];
+    cur = P.q_ray[i < n_low ? i : top - (i - n_low)];
     const uint32_t rec = cur >> 1;
     if (cur & 1u) {
       const F8 n23 = ld256(reinterpret_cast<const F8*>(&P.nee[rec].n2));
@@ -99,17 +102,29 @@ struct ConnectWork {
   }
 };
 
+// every ray of the round, or (closest_only) the closest-hit MIS rays when occlusion_kernel has traced the any-hit ones
 template <bool COUNT, bool DIST>
-__global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) connect_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ PathArrays P, RoundCounters* ctr, GlobalCounters* g) {
+__global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) connect_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ PathArrays P, uint32_t cap,
+                                                                           bool closest_only, RoundCounters* ctr, GlobalCounters* g) {
   uint32_t c_nodes = 0, c_tris = 0;
-  ConnectWork w{P, 0u, 0u, 0u};
-  trace_stream<COUNT, DIST>(sc, ctr->n_ray, &ctr->t_ray, w, &c_nodes, &c_tris);
+  const uint32_t n_low = closest_only ? 0u : ctr->n_ray;
+  ConnectWork w{P, n_low, 2u * cap - 1u, 0u, 0u, 0u};
+  trace_stream<COUNT, DIST>(sc, n_low + ctr->n_ray_closest, closest_only ? &ctr->t_ray_closest : &ctr->t_ray, w, &c_nodes, &c_tris);
   warp_sum_add(w.n_shadow, &g->shadow_rays);
   warp_sum_add(w.n_mis, &g->mis_rays);
   if (COUNT) {
     warp_sum_add(c_nodes, &g->nee_nodes_tested);
     warp_sum_add(c_tris, &g->nee_tris_tested);
   }
+}
+
+// the any-hit rays of the round over the occlusion tree
+__global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) occlusion_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ PathArrays P, RoundCounters* ctr, GlobalCounters* g) {
+  const uint32_t n = ctr->n_ray;
+  ConnectWork w{P, n, 0u, 0u, 0u, 0u};
+  trace_occlusion(sc, n, &ctr->t_ray, w);
+  warp_sum_add(w.n_shadow, &g->shadow_rays);
+  warp_sum_add(w.n_mis, &g->mis_rays);
 }
 
 // ---- standalone traversal kernels (ptrs_intersect*, the BVH microbenchmark) --------------------------
@@ -155,6 +170,12 @@ __global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) intersect_kernel(con
   }
 }
 
+__global__ void __launch_bounds__(128, PT_TRACE_MIN_BLOCKS) intersect_p_occlusion_kernel(const __grid_constant__ DevScene sc, const PtrsRay* __restrict__ rays, uint32_t n,
+                                                                                         uint8_t* __restrict__ occluded, uint32_t* ticket) {
+  IntersectWork w{rays, nullptr, occluded, true, nullptr};
+  trace_occlusion(sc, n, ticket, w);
+}
+
 // ---- launchers -----------------------------------------------------------------------------------------
 // <.., DIST>: front-to-back child order on trees the library built (DevScene::dist_order); the counted variants read the flag at
 // run time, so they exist once
@@ -164,17 +185,22 @@ void launch_extend(cudaStream_t st, int sm, bool count, const DevScene& sc, cons
   else if (sc.dist_order) extend_kernel<false, true><<<PT_GRID((extend_kernel<false, true>), 128, sm), 128, 0, st>>>(sc, P, q_ext, q_class, cap, ctr, g);
   else extend_kernel<false, false><<<PT_GRID((extend_kernel<false, false>), 128, sm), 128, 0, st>>>(sc, P, q_ext, q_class, cap, ctr, g);
 }
-void launch_connect(cudaStream_t st, int sm, bool count, const DevScene& sc, const PathArrays& P, RoundCounters* ctr, GlobalCounters* g) {
-  if (count) connect_kernel<true, false><<<PT_GRID((connect_kernel<true, false>), 128, sm), 128, 0, st>>>(sc, P, ctr, g);
-  else if (sc.dist_order) connect_kernel<false, true><<<PT_GRID((connect_kernel<false, true>), 128, sm), 128, 0, st>>>(sc, P, ctr, g);
-  else connect_kernel<false, false><<<PT_GRID((connect_kernel<false, false>), 128, sm), 128, 0, st>>>(sc, P, ctr, g);
+void launch_connect(cudaStream_t st, int sm, bool count, const DevScene& sc, const PathArrays& P, uint32_t cap, bool closest_only, RoundCounters* ctr,
+                    GlobalCounters* g) {
+  if (count) connect_kernel<true, false><<<PT_GRID((connect_kernel<true, false>), 128, sm), 128, 0, st>>>(sc, P, cap, closest_only, ctr, g);
+  else if (sc.dist_order) connect_kernel<false, true><<<PT_GRID((connect_kernel<false, true>), 128, sm), 128, 0, st>>>(sc, P, cap, closest_only, ctr, g);
+  else connect_kernel<false, false><<<PT_GRID((connect_kernel<false, false>), 128, sm), 128, 0, st>>>(sc, P, cap, closest_only, ctr, g);
+}
+void launch_occlusion(cudaStream_t st, int sm, const DevScene& sc, const PathArrays& P, RoundCounters* ctr, GlobalCounters* g) {
+  occlusion_kernel<<<PT_GRID(occlusion_kernel, 128, sm), 128, 0, st>>>(sc, P, ctr, g);
 }
 void launch_intersect(cudaStream_t st, int sm, bool any_hit, bool count, const DevScene& sc, const PtrsRay* rays, uint32_t n, PtrsHit* hits,
                       uint8_t* occluded, uint32_t* ticket, GlobalCounters* g, const uint32_t* prim_map) {
 #define PT_LAUNCH_INTERSECT(A, C, D) \
   intersect_kernel<A, C, D><<<PT_GRID((intersect_kernel<A, C, D>), 128, sm), 128, 0, st>>>(sc, rays, n, hits, occluded, ticket, g, prim_map)
   const bool dist = sc.dist_order != 0;
-  if (!any_hit && count) PT_LAUNCH_INTERSECT(false, true, false);
+  if (any_hit && !count && sc.n_wnodes > 0) intersect_p_occlusion_kernel<<<PT_GRID(intersect_p_occlusion_kernel, 128, sm), 128, 0, st>>>(sc, rays, n, occluded, ticket);
+  else if (!any_hit && count) PT_LAUNCH_INTERSECT(false, true, false);
   else if (any_hit && count) PT_LAUNCH_INTERSECT(true, true, false);
   else if (!any_hit && dist) PT_LAUNCH_INTERSECT(false, false, true);
   else if (!any_hit) PT_LAUNCH_INTERSECT(false, false, false);

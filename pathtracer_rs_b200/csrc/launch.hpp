@@ -38,7 +38,9 @@ void launch_ray_probe(cudaStream_t st, const RenderConst& rc, const uint32_t* so
 // k_trace.cu
 void launch_extend(cudaStream_t st, int sm, bool count, const DevScene& sc, const PathArrays& P, const int* q_ext, int* q_class, uint32_t cap,
                    RoundCounters* ctr, GlobalCounters* g);
-void launch_connect(cudaStream_t st, int sm, bool count, const DevScene& sc, const PathArrays& P, RoundCounters* ctr, GlobalCounters* g);
+void launch_connect(cudaStream_t st, int sm, bool count, const DevScene& sc, const PathArrays& P, uint32_t cap, bool closest_only, RoundCounters* ctr,
+                    GlobalCounters* g);
+void launch_occlusion(cudaStream_t st, int sm, const DevScene& sc, const PathArrays& P, RoundCounters* ctr, GlobalCounters* g);
 void launch_intersect(cudaStream_t st, int sm, bool any_hit, bool count, const DevScene& sc, const PtrsRay* rays, uint32_t n, PtrsHit* hits,
                       uint8_t* occluded, uint32_t* ticket, GlobalCounters* g, const uint32_t* prim_map);
 

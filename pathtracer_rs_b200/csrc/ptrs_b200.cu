@@ -198,6 +198,8 @@ struct PtrsScene {
   int device = 0;
   DevScene dev{};
   DevBuf<float4> nodes, tri_verts;
+  DevBuf<float4> wnodes;  // occlusion tree (dev_accel.cuh trace_occlusion), empty when the scene has none
+  bool has_area_light = false;  // closest-hit MIS rays exist only for area lights
   DevBuf<uint4> tri_index;
   DevBuf<float4> tri_shade;
   DevBuf<uint32_t> prim_map;  // device-built BVH: BVH position -> caller's primitive index
@@ -476,7 +478,17 @@ int32_t run_batch(PtrsScene* s, const RenderConst& rc, bool exact_shading, uint6
       tm.end();
       tm.begin(ST_CONNECT);
       if (s->dev.n_lights > 0) {
-        launch_connect(st, sm, s->count_visits, s->dev, P, c, w.gcount.p);
+        // any-hit rays over the occlusion tree, closest-hit MIS rays (area lights only) over the reference tree; in stats
+        // mode everything takes the reference walk, so that the visit counters stay the reference's
+        if (!s->count_visits && s->dev.n_wnodes > 0) {
+          launch_occlusion(st, sm, s->dev, P, c, w.gcount.p);
+          if (s->has_area_light) {
+            launch_connect(st, sm, false, s->dev, P, cap, true, c, w.gcount.p);
+            s->stats.launches += 1;
+          }
+        } else {
+          launch_connect(st, sm, s->count_visits, s->dev, P, cap, false, c, w.gcount.p);
+        }
         tm.end();
         tm.begin(ST_RESOLVE);
         launch_connect_resolve(st, sm, s->dev, P, w.q_nee.p, c);
@@ -517,6 +529,85 @@ int32_t ptrs_device_count(int32_t* count) {
 int32_t ptrs_set_device(int32_t device) {
   CUDA_TRY(cudaSetDevice(device));
   return PTRS_OK;
+}
+
+// The occlusion tree (dev_accel.cuh, trace_occlusion) collapsed from the reference's flattened tree (depth-first preorder,
+// first child at i + 1, second at `offset`).  Greedy: a wide node starts from the two children of a reference interior node
+// and, while it has fewer than four slots, replaces the interior slot of largest surface area by its two children.  Any
+// collapse is exact; this choice only favours speed.  Returns false, and the scene traces its any-hit rays over the
+// reference tree, when the tree cannot be collapsed exactly: an interior box that does not contain a child's box (the
+// reference builder never makes one), or a leaf the 4-byte child word cannot hold (more than 16 primitives, or primitives
+// beyond 2^27).
+static bool build_occlusion_tree(const PtrsBvhNode* nodes, uint32_t n_nodes, std::vector<float4>* out) {
+  auto contains = [&](const PtrsBvhNode& a, const PtrsBvhNode& b) {
+    for (int k = 0; k < 3; ++k)
+      if (!(a.bounds_min[k] <= b.bounds_min[k]) || !(a.bounds_max[k] >= b.bounds_max[k])) return false;
+    return true;
+  };
+  for (uint32_t i = 0; i < n_nodes; ++i) {
+    const PtrsBvhNode& n = nodes[i];
+    if (n.n_prims > 0) {
+      if (n.n_prims > 16 || (uint64_t)n.offset + n.n_prims > (1u << 27)) return false;
+    } else if (!contains(n, nodes[i + 1]) || !contains(n, nodes[n.offset])) {
+      return false;
+    }
+  }
+  auto area = [&](uint32_t i) {
+    const PtrsBvhNode& n = nodes[i];
+    const float dx = n.bounds_max[0] - n.bounds_min[0], dy = n.bounds_max[1] - n.bounds_min[1], dz = n.bounds_max[2] - n.bounds_min[2];
+    return dx * dy + dy * dz + dz * dx;
+  };
+  out->clear();
+  std::vector<std::pair<uint32_t, uint32_t>> todo{{0u, 0u}};  // (reference node, wide node)
+  out->resize(8);
+  while (!todo.empty()) {
+    const auto [r, w] = todo.back();
+    todo.pop_back();
+    std::vector<uint32_t> slot;
+    if (nodes[r].n_prims > 0) slot.push_back(r);  // a single-leaf tree: its root alone
+    else slot = {r + 1, nodes[r].offset};
+    while (slot.size() < 4) {
+      int best = -1;
+      for (int k = 0; k < (int)slot.size(); ++k)
+        if (nodes[slot[k]].n_prims == 0 && (best < 0 || area(slot[k]) > area(slot[best]))) best = k;
+      if (best < 0) break;
+      const uint32_t c = slot[best];
+      slot[best] = c + 1;
+      slot.push_back(nodes[c].offset);
+    }
+    float lo[3][4], hi[3][4];
+    uint32_t child[4];
+    for (int k = 0; k < 4; ++k) {
+      if (k >= (int)slot.size()) {  // empty slot: an empty box and the word PT_W_NONE
+        for (int a = 0; a < 3; ++a) {
+          lo[a][k] = INFINITY;
+          hi[a][k] = -INFINITY;
+        }
+        child[k] = PT_W_NONE;
+        continue;
+      }
+      const PtrsBvhNode& n = nodes[slot[k]];
+      for (int a = 0; a < 3; ++a) {
+        lo[a][k] = n.bounds_min[a];
+        hi[a][k] = n.bounds_max[a];
+      }
+      if (n.n_prims > 0) {
+        child[k] = PT_W_LEAF_BIT | ((uint32_t)(n.n_prims - 1) << 27) | n.offset;
+      } else {
+        child[k] = (uint32_t)(out->size() / 8);
+        todo.emplace_back(slot[k], child[k]);
+        out->resize(out->size() + 8);
+      }
+    }
+    float4* rec = out->data() + 8 * (size_t)w;
+    for (int a = 0; a < 3; ++a) {
+      rec[2 * a] = make_float4(lo[a][0], lo[a][1], lo[a][2], lo[a][3]);
+      rec[2 * a + 1] = make_float4(hi[a][0], hi[a][1], hi[a][2], hi[a][3]);
+    }
+    std::memcpy(&rec[6], child, 16);
+    rec[7] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  return true;
 }
 
 static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsScene** out) {
@@ -692,6 +783,13 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
       s->nodes.p = nodes;
       s->nodes.n = (size_t)n_dev_nodes * 2;
       s->scene_bytes += (uint64_t)n_dev_nodes * 32;
+      // device-built scenes keep the reference walk for any-hit rays: their tree is not the reference's, and the
+      // collapse works on the caller's records here on the host
+      std::vector<float4> wide;
+      if (build_occlusion_tree(d->nodes, d->n_nodes, &wide)) {
+        CUDA_TRY(s->wnodes.upload(wide.data(), wide.size()));
+        s->scene_bytes += (uint64_t)wide.size() * 16;
+      }
       launch_assemble_tris(0, d->n_prims, nullptr, pv.p, pos.p, pm.p, pmat.p, pal.p, s->meshes.p, s->tri_verts.p, s->tri_index.p, nullptr);
       CUDA_TRY(cudaGetLastError());
       CUDA_TRY(cudaStreamSynchronize(0));  // the staging buffers above are released when this scope ends
@@ -884,6 +982,9 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
   v.dist_order = device_bvh ? 1u : 0u;
   if (const char* e = std::getenv("PTRS_DIST_ORDER")) v.dist_order = device_bvh && std::atoi(e) != 0;  // tuning only
   if (const char* e = std::getenv("PTRS_BOX_MIN")) v.box_min = (uint32_t)std::max(1, std::min(32, std::atoi(e)));  // tuning only
+  v.wnodes = s->wnodes.p;
+  v.n_wnodes = d->n_prims > 0 ? (uint32_t)(s->wnodes.n / 8) : 0u;
+  for (uint32_t i = 0; i < d->n_lights; ++i) s->has_area_light |= d->lights[i].type == PTRS_LIGHT_AREA;
   v.uses_differentials = 0;
   for (uint32_t i = 0; i < d->n_materials; ++i) {
     static const int n_tex[PTRS_MAT_COUNT] = {1, 0, 3, 5, 4, 4};

@@ -75,7 +75,7 @@ struct PathArrays {
   float4* q_hit;    // PT_N_CLASSES x cap, aligned with the class queues
   NeeRec* nee;      // cap, aligned with the connect queue
   NeeRes* nee_res;  // cap, aligned with the connect queue
-  uint32_t* q_ray;  // 2 x cap: the rays the connect stage has to trace, 2 * record + {0 shadow segment, 1 MIS ray}
+  uint32_t* q_ray;  // 2 x cap: the rays the connect stage has to trace, 2 * record + {0 shadow segment, 1 MIS ray} (RoundCounters)
 };
 #define PT_F_SPECULAR (1u << 16)
 #define PT_F_HAS_DIFF (1u << 17)
@@ -131,9 +131,12 @@ struct RoundCounters {
   uint32_t n_class[PT_N_CLASSES];  // lengths of the per-material shade queues
   // connect stage: direct-lighting records and the rays of those records (q_ray).  The pair is one 8-byte
   // aligned word so that shade reserves both with a single 64-bit atomicAdd (records in the low half).
+  // n_ray counts the any-hit rays at the bottom of q_ray, n_ray_closest the closest-hit MIS rays at its top
+  // (q_ray[2 * cap - 1 - j]); the two never meet, every record has at most two rays
   uint32_t n_nee, n_ray;
   uint32_t t_ext, t_class[PT_N_CLASSES], t_nee, t_ray;  // work tickets
-  uint32_t pad[32 - 6 - 2 * PT_N_CLASSES];  // 128 B per round
+  uint32_t n_ray_closest, t_ray_closest;
+  uint32_t pad[32 - 8 - 2 * PT_N_CLASSES];  // 128 B per round
 };
 static_assert(offsetof(RoundCounters, n_nee) % 8 == 0 && sizeof(RoundCounters) == 128, "RoundCounters layout");
 
