@@ -48,7 +48,7 @@ $(OBJ)/k_shade_exact_%.o: $(CS)/k_shade.cu $(DEV_HDRS)
 
 $(OBJ)/k_shade_%.o: $(CS)/k_shade.cu $(DEV_HDRS)
 	@mkdir -p $(OBJ)
-	$(NVCC) $(SHADEFLAGS) $(SHADE_EXTRA) -DPT_SHADE_MAT=$* -c $< -o $@ > $(OBJ)/k_shade_$*.ptxas.log 2>&1 || (cat $(OBJ)/k_shade_$*.ptxas.log; false)
+	$(NVCC) $(SHADEFLAGS) -DPT_SHADE_MAT=$* -c $< -o $@ > $(OBJ)/k_shade_$*.ptxas.log 2>&1 || (cat $(OBJ)/k_shade_$*.ptxas.log; false)
 
 $(OBJ)/sobol_blob.o: $(CS)/sobol_blob.S $(BLOB)
 	@mkdir -p $(OBJ)

@@ -171,44 +171,20 @@ PT_DEV float fmin3_nn(float a, float b, float c) {
   return r;
 }
 
-// Two node records in ONE asm statement: both loads are issued before anything waits on the first (left to itself the
-// register allocator may give the second load the registers the first record's slab test is still reading, which
-// serialises two DRAM round trips per traversal step: measured +17 % on the 10 M-triangle tree with incoherent rays).
-#ifndef PT_PAIR_LOAD128
-#define PT_PAIR_LOAD128 1
-#endif
-#ifndef PT_NODE_EVICT_LAST
-#define PT_NODE_EVICT_LAST 0
-#endif
+// Two node records, both in flight before anything waits on the first (left to itself the register allocator may give the
+// second load the registers the first record's slab test is still reading, which serialises two DRAM round trips per
+// traversal step: measured +17 % on the 10 M-triangle tree with incoherent rays).
 PT_DEV void load_node_pair(const float4* __restrict__ nodes, uint32_t ia, uint32_t ib, NodeLoad* a, NodeLoad* b) {
-#if PT_PAIR_LOAD128
   // four 128-bit loads, the first half of either record first: with 64 registers per thread the allocator keeps three of
   // them in flight and re-uses the first one's registers for the fourth — which by then is an L1 hit, because the two
   // halves of a 32-byte record are one sector.  Two 256-bit loads get serialised instead (the second one is given the
   // registers the first record's slab test is still reading): two DRAM round trips per step on trees beyond L2 size.
   const float4* pa = nodes + 2 * (size_t)ia;
   const float4* pb = nodes + 2 * (size_t)ib;
-#if PT_NODE_EVICT_LAST
-  // node lines are asked to stay: the second half of a record may be read a few dozen instructions after the first
-  auto ld = [](const float4* p) {
-    float4 v;
-    asm("ld.global.nc.L1::evict_last.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    return v;
-  };
-  a->a = ld(pa);
-  b->a = ld(pb);
-  a->b = ld(pa + 1);
-  b->b = ld(pb + 1);
-#else
   a->a = __ldg(pa);
   b->a = __ldg(pb);
   a->b = __ldg(pa + 1);
   b->b = __ldg(pb + 1);
-#endif
-#else
-  *a = load_node(nodes, ia);
-  *b = load_node(nodes, ib);
-#endif
 }
 
 // bounds.rs:190-232.  The slab arithmetic does not depend on the ray's current t_max except for the
@@ -280,21 +256,23 @@ PT_DEV void box_geom_pair(const NodeLoad& a, const NodeLoad& b, V3 o, V3 inv_dir
 // A warp owns 32 ray slots.  Each lane takes ITS ray through the box-test / triangle-test decisions of
 // accelerator.rs:359-475, with:
 //   refill     lanes whose ray has ended pull new work items with ONE atomicAdd for the whole warp
-//              (persistent threads, warp-aggregated fetch) as soon as PT_REFILL_IDLE lanes are idle
+//              (persistent threads, warp-aggregated fetch) as soon as PT_REFILL_IDLE lanes are idle (warp_refill)
 //   expand     a lane standing on an interior node loads BOTH children and runs both slab tests.  The
 //              near child (dir_is_neg[axis]) is accepted against t_max; the far child's entry distance goes
 //              on the stack, and `t_entry < t_max` is applied again when it is popped — the very test the
 //              reference performs at that moment, since only that comparison depends on t_max
-//   postpone   (fast variant) a lane that reaches a leaf parks it and keeps descending until it holds a
-//              second leaf; the warp switches to the triangle phase when fewer than box_min (DevScene, 12 or 20) lanes can
-//              still take a box step.  Exactness: with nested boxes the slab entry distance can only grow
+//   postpone   (trace_fast) a lane that reaches a leaf parks it and keeps descending until it holds a
+//              second leaf; the warp takes PT_BOX_STEPS box steps per scheduling decision and switches to the
+//              triangle phase when fewer than box_min (DevScene, 12 or 20) lanes can still take a box step, where
+//              each lane tests one triangle per step.  Exactness: with nested boxes the slab entry distance can only grow
 //              from a node to its descendants (float subtraction and multiplication are monotonic), so a
 //              node accepted under a stale (larger) t_max that the reference would have culled can only
 //              lead to leaves whose own entry distance fails the CURRENT t_max — and every parked node is
 //              re-validated with `t_entry < t_max` whenever a hit shrinks t_max, every stack entry when
 //              it is popped.  Leaves are processed first-in first-out, so each triangle is tested in the
 //              reference's order against the reference's t_max: hits, ties and barycentrics are identical.
-// Stack entries are 16 B {entry distance, offset, n_prims | axis << 16, -}: a pop needs no node reload.
+// Stack entries are 16 B {entry distance, offset, n_prims | axis << 16, -}: a pop needs no node reload.  A ray pushes at
+// most one entry per level it descends, and ptrs_scene_create refuses trees deeper than the PT_STACK_SIZE entries.
 //
 // Work is a functor object with
 //   bool begin(uint32_t item, LaneRay* r)                       first ray of a work item (false: nothing to trace)
@@ -306,12 +284,32 @@ struct LaneRay {
   bool any_hit;
 };
 
-#ifndef PT_REFILL_IDLE
 #define PT_REFILL_IDLE 8
-#endif
-#ifndef PT_SEARCH_MIN
 #define PT_SEARCH_MIN 6
-#endif
+
+// The engine's refill step (above), shared by the three streaming walks; start(r) is called for each lane that got a ray.
+template <class Work, class Start>
+PT_DEV void warp_refill(bool idle_lane, uint32_t n_items, uint32_t* ticket, bool* exhausted, Work& work, uint32_t* item, Start&& start) {
+  const uint32_t idle = __ballot_sync(0xffffffffu, idle_lane);
+  if (!*exhausted && (__popc(idle) >= PT_REFILL_IDLE)) {
+    const int lane = threadIdx.x & 31;
+    const int leader = __ffs(idle) - 1;
+    uint32_t base = 0;
+    if (lane == leader) base = atomicAdd(ticket, (uint32_t)__popc(idle));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (base + (uint32_t)__popc(idle) >= n_items) *exhausted = true;
+    if (idle_lane) {
+      const uint32_t i = base + (uint32_t)__popc(idle & ((1u << lane) - 1u));
+      if (i < n_items) {
+        LaneRay r;
+        if (work.begin(i, &r)) {
+          *item = i;
+          start(r);
+        }
+      }
+    }
+  }
+}
 
 // empty accelerator: every ray misses (accelerator.rs:360-362)
 template <class Work>
@@ -345,49 +343,8 @@ PT_DEV void trace_empty(uint32_t n_items, uint32_t* ticket, Work& work) {
 #define PT_RB_LIVE 64u
 // box steps per scheduling decision (measured on B200, round 2: 1 -> 3 steps takes 3 % off the traversal kernels on every
 // scene; 4 is level with 3)
-#ifndef PT_BOX_STEPS
 #define PT_BOX_STEPS 3
-#endif
-#ifndef PT_TRI_STEPS
-#define PT_TRI_STEPS 1
-#endif
-// PT_EAGER_POP: a lane that is left without a node pops its next stack entry at the END of the step (one predicated
-// 16-byte local load in the convergent instruction stream) and the entry's `t_entry < t_max` test — the reference's box
-// test at pop time — is made when the node is used, together with the re-validation every node in hand needs anyway after
-// a hit has shrunk t_max.  Replaces the divergent pop section at the top of the step.
-#ifndef PT_EAGER_POP
-#define PT_EAGER_POP 0
-#endif
-#ifndef PT_NEAR_LEAF_DIRECT
-#define PT_NEAR_LEAF_DIRECT 0
-#endif
-// PT_SMEM_STACK = K: the K entries nearest the bottom of every ray's pending stack live in shared memory, one 16-byte
-// column per thread ([level][thread], so a warp's access is conflict-free whatever levels its lanes stand on: four
-// wavefronts, where the same access to thread-interleaved local memory touches four 128-byte lines PER DISTINCT LEVEL
-// among the lanes); deeper entries stay in local memory.  Blocks of PT_TRACE_BLOCK threads.
-#ifndef PT_SMEM_STACK
-#define PT_SMEM_STACK 0
-#endif
-#ifndef PT_STACK8
-#define PT_STACK8 0
-#endif
-#ifndef PT_PUSH_PREFETCH
-#define PT_PUSH_PREFETCH 0
-#endif
-// PT_PARK_PREFETCH_ON: when a leaf is parked its first triangle is requested into L1 — unlike a pushed node a parked leaf is
-// always processed, and until then the lane keeps taking box steps
-#ifndef PT_PARK_PREFETCH_ON
-#define PT_PARK_PREFETCH_ON 0
-#endif
-#if PT_PARK_PREFETCH_ON
-#define PT_PARK_PREFETCH(prim) asm volatile("prefetch.global.L1 [%0];" ::"l"(sc.tri_verts + 3 * (size_t)(prim)))
-#else
-#define PT_PARK_PREFETCH(prim) ((void)0)
-#endif
 
-#ifndef PT_TRACE_BLOCK
-#define PT_TRACE_BLOCK 128
-#endif
 // DIST: of two entered children the one the ray enters first is visited first (trees the library built itself) instead of
 // dir_is_neg[axis] (the reference's order on the reference's tree).  A template parameter, so that the reference path's
 // code is untouched.
@@ -403,52 +360,6 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
   const int box_min = (int)sc.box_min;
   const bool pop_twice = sc.pop_twice != 0;
   constexpr bool dist_order = DIST;
-#if PT_STACK8
-  // 8-byte entries {entry distance, packed node}: half the local-memory footprint of the 1024 stacks per SM, which is what
-  // matters when the tree itself does not fit in L2 and the stacks compete with its nodes for L1.  Packed node word:
-  //   bit 31 = 0              interior: first child slot (even, < 2^30) << 1 | split axis
-  //   bit 31 = 1, bit 30 = 0  leaf: (n_prims - 1) << 26 | first primitive      (n_prims <= 16, primitive < 2^26)
-  //   bit 31 = 1, bit 30 = 1  leaf by reference: the node's slot; (offset, n_prims) are re-read when it is popped
-  uint2 stack[PT_STACK_SIZE];
-  auto st_load = [&](int i, float* t, uint32_t* off, uint32_t* meta) {
-    const uint2 e = stack[i];
-    *t = __uint_as_float(e.x);
-    const uint32_t w = e.y;
-    if (!(w & 0x80000000u)) {
-      *off = (w & ~3u) >> 1;
-      *meta = (w & 3u) << 16;
-    } else if (!(w & 0x40000000u)) {
-      *off = w & 0x03ffffffu;
-      *meta = ((w >> 26) & 15u) + 1u;
-    } else {
-      const float2 om = __ldg(reinterpret_cast<const float2*>(sc.nodes + 2 * (size_t)(w & 0x3fffffffu) + 1) + 1);
-      *off = __float_as_uint(om.x);
-      *meta = __float_as_uint(om.y);
-    }
-  };
-  auto st_store = [&](int i, float t, uint32_t off, uint32_t meta, uint32_t slot) {
-    const uint32_t np = meta & 0xffffu;
-    uint32_t w;
-    if (np == 0u) w = (off << 1) | ((meta >> 16) & 3u);
-    else if (np <= 16u && off < (1u << 26)) w = 0x80000000u | ((np - 1u) << 26) | off;
-    else w = 0xc0000000u | slot;
-    stack[i] = make_uint2(__float_as_uint(t), w);
-  };
-#elif PT_SMEM_STACK
-  __shared__ uint4 sm_stack[PT_SMEM_STACK * PT_TRACE_BLOCK];
-  uint4 stack[PT_STACK_SIZE - PT_SMEM_STACK];
-  auto st_load = [&](int i, float* t, uint32_t* off, uint32_t* meta) {
-    const uint4 e = i < PT_SMEM_STACK ? sm_stack[i * PT_TRACE_BLOCK + threadIdx.x] : stack[i - PT_SMEM_STACK];
-    *t = __uint_as_float(e.x);
-    *off = e.y;
-    *meta = e.z;
-  };
-  auto st_store = [&](int i, float t, uint32_t off, uint32_t meta, uint32_t) {
-    const uint4 e = make_uint4(__float_as_uint(t), off, meta, 0u);
-    if (i < PT_SMEM_STACK) sm_stack[i * PT_TRACE_BLOCK + threadIdx.x] = e;
-    else stack[i - PT_SMEM_STACK] = e;
-  };
-#else
   uint4 stack[PT_STACK_SIZE];
   auto st_load = [&](int i, float* t, uint32_t* off, uint32_t* meta) {
     const uint4 e = stack[i];
@@ -456,8 +367,9 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
     *off = e.y;
     *meta = e.z;
   };
+  // (the last argument, the pushed child's node slot, is not stored: without it nvcc 12.9 inverts the predicate of the
+  // child selects in the DIST kernels — same instructions, different machine code)
   auto st_store = [&](int i, float t, uint32_t off, uint32_t meta, uint32_t) { stack[i] = make_uint4(__float_as_uint(t), off, meta, 0u); };
-#endif
   int sp_ = 0;
   // node in hand (its box test passed under the t_max current at that time): offset, meta, entry distance
   uint32_t cur_off = 0, cur_meta = PT_NO_NODE;
@@ -499,116 +411,13 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
   };
 
   for (;;) {
-    // ---- refill ------------------------------------------------------------------------------------
-    const uint32_t idle = __ballot_sync(FULL, !(rbits & PT_RB_LIVE));
-    if (!exhausted && (__popc(idle) >= PT_REFILL_IDLE)) {
-      const int lane = threadIdx.x & 31;
-      const int leader = __ffs(idle) - 1;
-      uint32_t base = 0;
-      if (lane == leader) base = atomicAdd(ticket, (uint32_t)__popc(idle));
-      base = __shfl_sync(FULL, base, leader);
-      if (base + (uint32_t)__popc(idle) >= n_items) exhausted = true;
-      if (!(rbits & PT_RB_LIVE)) {
-        const uint32_t i = base + (uint32_t)__popc(idle & ((1u << lane) - 1u));
-        if (i < n_items) {
-          LaneRay r;
-          if (work.begin(i, &r)) {
-            item = i;
-            start_ray(r);
-          }
-        }
-      }
-    }
+    warp_refill(!(rbits & PT_RB_LIVE), n_items, ticket, &exhausted, work, &item, start_ray);
     if (__ballot_sync(FULL, rbits & PT_RB_LIVE) == 0) {
       if (exhausted) break;
       continue;
     }
 
     // ---- box phase: pop / park / expand ----------------------------------------------------------------
-#if PT_EAGER_POP
-    auto eager_pop = [&]() {
-      if ((rbits & PT_RB_LIVE) && cur_meta == PT_NO_NODE && sp_ > 0) {
-        --sp_;
-        st_load(sp_, &cur_t, &cur_off, &cur_meta);
-      }
-    };
-    auto box_step = [&]() {
-      const bool live = (rbits & PT_RB_LIVE) != 0;
-      // the node in hand under the current t_max: the reference's box test at pop time, and the re-test a node accepted
-      // before a hit needs
-      if (cur_meta != PT_NO_NODE && !(cur_t < t_max)) cur_meta = PT_NO_NODE;
-#if PT_EAGER_POP == 2
-      // the entry popped ahead was culled: one more pop, tested on the spot, so that the lane still expands a node in this step
-      if (live && cur_meta == PT_NO_NODE && sp_ > 0) {
-        --sp_;
-        float et;
-        uint32_t eo, em;
-        st_load(sp_, &et, &eo, &em);
-        if (et < t_max) {
-          cur_t = et;
-          cur_off = eo;
-          cur_meta = em;
-        }
-      }
-#endif
-      if (live && cur_meta != PT_NO_NODE) {
-        if ((cur_meta & 0xffffu) != 0) {
-          if (pl_cnt == 0) {  // park the leaf, keep descending
-            pl_off = cur_off;
-            pl_cnt = cur_meta & 0xffffu;
-            cur_meta = PT_NO_NODE;
-          }
-        } else {
-          const NodeLoad L = load_node(sc.nodes, cur_off);
-          const NodeLoad R = load_node(sc.nodes, cur_off + 1);
-          const bool nx = rbits & PT_RB_NX, ny = rbits & PT_RB_NY, nz = rbits & PT_RB_NZ;
-          float tl, tr;
-          const bool gl = box_geom(L, o, inv_dir, nx, ny, nz, &tl);
-          const bool gr = box_geom(R, o, inv_dir, nx, ny, nz, &tr);
-          const bool neg = dist_order ? (tr < tl) : (((rbits >> ((cur_meta >> 16) & 3u)) & 1u) != 0);  // dir_is_neg[axis], or nearer child first
-          // near child first (accelerator.rs:393-404)
-          const bool gn = neg ? gr : gl, gf = neg ? gl : gr;
-          const float tn = neg ? tr : tl, tf = neg ? tl : tr;
-          const float4 nb = neg ? R.b : L.b, fb = neg ? L.b : R.b;
-          bool an = gn && tn < t_max;
-          const bool af = gf && tf < t_max;
-          // an entered near child that is a leaf goes straight to the free parking slot; the far child is then the node
-          // in hand without a push / pop pair
-          if (an && (__float_as_uint(nb.w) & 0xffffu) != 0u && pl_cnt == 0u) {
-            pl_off = __float_as_uint(nb.z);
-            pl_cnt = __float_as_uint(nb.w) & 0xffffu;
-            an = false;
-          }
-          if (af && !an) {
-            cur_t = tf;
-            cur_off = __float_as_uint(fb.z);
-            cur_meta = __float_as_uint(fb.w);
-          } else {
-            if (af) {
-              if (sp_ < PT_STACK_SIZE) {  // always true: ptrs_scene_create refuses trees deeper than the stack
-                st_store(sp_, tf, __float_as_uint(fb.z), __float_as_uint(fb.w), cur_off + (neg ? 0u : 1u));
-                ++sp_;
-              }
-            }
-            if (an) {
-              cur_t = tn;
-              cur_off = __float_as_uint(nb.z);
-              cur_meta = __float_as_uint(nb.w);
-            } else {
-              cur_meta = PT_NO_NODE;
-            }
-          }
-          // the node now in hand is a leaf and the parking slot is free: park it here instead of in the next iteration
-          if (cur_meta != PT_NO_NODE && (cur_meta & 0xffffu) != 0u && pl_cnt == 0u) {
-            pl_off = cur_off;
-            pl_cnt = cur_meta & 0xffffu;
-            cur_meta = PT_NO_NODE;
-          }
-        }
-      }
-      eager_pop();
-    };
-#else
     // (a lane without a ray has no node in hand, an empty stack and no parked leaf, so none of the tests below asks for
     // PT_RB_LIVE on top)
     auto box_step = [&]() {
@@ -631,7 +440,6 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
             // (scheduling only; DevScene::pop_twice)
             if (PT_IS_LEAF(cur_meta) && pl_cnt == 0u) {
               pl_off = cur_off;
-              PT_PARK_PREFETCH(cur_off);
               pl_cnt = cur_meta & 0xffffu;
               cur_meta = PT_NO_NODE;
             }
@@ -650,7 +458,6 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
           if ((cur_meta & 0xffffu) != 0) {
             if (pl_cnt == 0) {  // park the leaf, keep descending
               pl_off = cur_off;
-              PT_PARK_PREFETCH(cur_off);
               pl_cnt = cur_meta & 0xffffu;
               cur_meta = PT_NO_NODE;
             }
@@ -673,17 +480,8 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
             const bool gn = swap ? gb : ga, gf = swap ? ga : gb;
             const float tn = swap ? tb : ta, tf = swap ? ta : tb;
             const float4 nb = swap ? B.b : A.b, fb = swap ? A.b : B.b;
-            bool an = gn && tn < t_max;
+            const bool an = gn && tn < t_max;
             const bool af = gf && tf < t_max;
-#if PT_NEAR_LEAF_DIRECT
-            // an entered near child that is a leaf goes straight to the free parking slot; the far child is then the node in
-            // hand without a push / pop pair
-            if (an && (__float_as_uint(nb.w) & 0xffffu) != 0u && pl_cnt == 0u) {
-              pl_off = __float_as_uint(nb.z);
-              pl_cnt = __float_as_uint(nb.w) & 0xffffu;
-              an = false;
-            }
-#endif
             if (af && !an) {
               // near child rejected, far child entered: the reference pushes the far child and pops it straight away; the
               // pop's re-test against t_max is what the node in hand gets anyway whenever a hit shrinks t_max
@@ -695,19 +493,6 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
                 if (sp_ < PT_STACK_SIZE) {  // always true: ptrs_scene_create refuses trees deeper than the stack
                   st_store(sp_, tf, __float_as_uint(fb.z), __float_as_uint(fb.w), cur_off + (neg ? 0u : 1u));
                   ++sp_;
-#if PT_PUSH_PREFETCH
-                  // the pushed child's own children (or its first triangle): requested now, so that the pop finds them in
-                  // L1 / L2 instead of starting the round trip then
-                  {
-                    const uint32_t fo = __float_as_uint(fb.z);
-                    const void* pf = (__float_as_uint(fb.w) & 0xffffu) ? (const void*)(sc.tri_verts + 3 * (size_t)fo) : (const void*)(sc.nodes + 2 * (size_t)fo);
-#if PT_PUSH_PREFETCH == 2
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(pf));
-#else
-                    asm volatile("prefetch.global.L1 [%0];" ::"l"(pf));
-#endif
-                  }
-#endif
                 }
               }
               if (an) {
@@ -721,7 +506,6 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
             // the node now in hand is a leaf and the parking slot is free: park it here instead of in the next iteration
             if (PT_IS_LEAF(cur_meta) && pl_cnt == 0u) {
               pl_off = cur_off;
-              PT_PARK_PREFETCH(cur_off);
               pl_cnt = cur_meta & 0xffffu;
               cur_meta = PT_NO_NODE;
             }
@@ -729,15 +513,10 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
         }
       }
     };
-#endif
     for (;;) {
       const bool live = (rbits & PT_RB_LIVE) != 0;
       const bool cur_leaf = PT_IS_LEAF(cur_meta);
-#if PT_EAGER_POP
-      const bool can_box = live && cur_meta != PT_NO_NODE && (!cur_leaf || pl_cnt == 0);  // no node in hand => empty stack
-#else
       const bool can_box = PT_IS_INTERIOR(cur_meta) || (cur_meta == PT_NO_NODE && sp_ > 0) || (cur_leaf && pl_cnt == 0);
-#endif
       const uint32_t bmask = __ballot_sync(FULL, can_box);
       if (bmask == 0) break;
       if (__popc(bmask) < box_min && __ballot_sync(FULL, live && !can_box) != 0) break;
@@ -748,22 +527,11 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
 
     // ---- triangle phase: parked leaves, first in first out -----------------------------------------------
     auto tri_step = [&]() {
-#if PT_EAGER_POP
-      const bool live = (rbits & PT_RB_LIVE) != 0;
-      if (live && pl_cnt == 0 && cur_meta != PT_NO_NODE && (cur_meta & 0xffffu) != 0) {  // second leaf moves up, if it still qualifies
-        if (cur_t < t_max) {
-          pl_off = cur_off;
-          pl_cnt = cur_meta & 0xffffu;
-        }
-        cur_meta = PT_NO_NODE;
-      }
-#else
       if (pl_cnt == 0 && PT_IS_LEAF(cur_meta)) {  // second leaf moves up
         pl_off = cur_off;
         pl_cnt = cur_meta & 0xffffu;
         cur_meta = PT_NO_NODE;
       }
-#endif
       if (pl_cnt != 0) {
         const uint32_t prim = pl_off;
         const float4 v0 = __ldg(sc.tri_verts + 3 * (size_t)prim);
@@ -788,23 +556,16 @@ PT_DEV void trace_fast(const DevScene& sc, uint32_t n_items, uint32_t* ticket, W
             pl_cnt = 0;
             sp_ = 0;
             cur_meta = PT_NO_NODE;
-          }
-#if !PT_EAGER_POP
-          else if (cur_meta != PT_NO_NODE && !(cur_t < t_max)) {
+          } else if (cur_meta != PT_NO_NODE && !(cur_t < t_max)) {
             cur_meta = PT_NO_NODE;  // the node in hand was accepted under the old t_max: re-validate
           }
-#endif
         }
       }
-#if PT_EAGER_POP
-      eager_pop();
-#endif
     };
     for (;;) {
       const bool has = pl_cnt != 0 || PT_IS_LEAF(cur_meta);
       if (__ballot_sync(FULL, has) == 0) break;
-#pragma unroll
-      for (int rep = 0; rep < PT_TRI_STEPS; ++rep) tri_step();
+      tri_step();
     }
 
     // ---- rays that ran out of nodes --------------------------------------------------------------------
@@ -831,8 +592,6 @@ PT_DEV void trace_counted(const DevScene& sc, uint32_t n_items, uint32_t* ticket
     return;
   }
   const uint32_t FULL = 0xffffffffu;
-  const int lane = threadIdx.x & 31;
-  const uint32_t lane_lt = (1u << lane) - 1u;
   uint4 stack[PT_STACK_SIZE];
   int sp_ = 0;
   uint32_t cur_off = 0, cur_meta = PT_NO_NODE;
@@ -875,25 +634,10 @@ PT_DEV void trace_counted(const DevScene& sc, uint32_t n_items, uint32_t* ticket
   };
 
   for (;;) {
-    const uint32_t idle = __ballot_sync(FULL, !active);
-    if (!exhausted && (__popc(idle) >= PT_REFILL_IDLE)) {
-      const int leader = __ffs(idle) - 1;
-      uint32_t base = 0;
-      if (lane == leader) base = atomicAdd(ticket, (uint32_t)__popc(idle));
-      base = __shfl_sync(FULL, base, leader);
-      if (base + (uint32_t)__popc(idle) >= n_items) exhausted = true;
-      if (!active) {
-        const uint32_t i = base + (uint32_t)__popc(idle & lane_lt);
-        if (i < n_items) {
-          LaneRay r;
-          if (work.begin(i, &r)) {
-            item = i;
-            active = true;
-            start_ray(r);
-          }
-        }
-      }
-    }
+    warp_refill(!active, n_items, ticket, &exhausted, work, &item, [&](const LaneRay& r) {
+      active = true;
+      start_ray(r);
+    });
     if (__ballot_sync(FULL, active) == 0) {
       if (exhausted) break;
       continue;
@@ -1046,26 +790,7 @@ PT_DEV void trace_occlusion(const DevScene& sc, uint32_t n_items, uint32_t* tick
   };
 
   for (;;) {
-    // ---- refill ------------------------------------------------------------------------------------
-    const uint32_t idle = __ballot_sync(FULL, !(rbits & PT_RB_LIVE));
-    if (!exhausted && (__popc(idle) >= PT_REFILL_IDLE)) {
-      const int lane = threadIdx.x & 31;
-      const int leader = __ffs(idle) - 1;
-      uint32_t base = 0;
-      if (lane == leader) base = atomicAdd(ticket, (uint32_t)__popc(idle));
-      base = __shfl_sync(FULL, base, leader);
-      if (base + (uint32_t)__popc(idle) >= n_items) exhausted = true;
-      if (!(rbits & PT_RB_LIVE)) {
-        const uint32_t i = base + (uint32_t)__popc(idle & ((1u << lane) - 1u));
-        if (i < n_items) {
-          LaneRay r;
-          if (work.begin(i, &r)) {
-            item = i;
-            start_ray(r);
-          }
-        }
-      }
-    }
+    warp_refill(!(rbits & PT_RB_LIVE), n_items, ticket, &exhausted, work, &item, start_ray);
     if (__ballot_sync(FULL, rbits & PT_RB_LIVE) == 0) {
       if (exhausted) break;
       continue;

@@ -8,11 +8,7 @@
 #include <stdint.h>
 
 #define PT_DEV __device__ __forceinline__
-#ifdef PT_INLINE_ALL
-#define PT_DEVN __device__ __forceinline__
-#else
 #define PT_DEVN static __device__ __noinline__
-#endif
 
 namespace ptrs {
 

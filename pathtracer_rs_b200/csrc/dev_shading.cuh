@@ -40,9 +40,6 @@ struct SurfInter {  // the fields of SurfaceMediumInteraction the path integrato
   int prim;
 };
 
-#ifndef PT_PACKED_SHADING
-#define PT_PACKED_SHADING 1
-#endif
 struct __align__(32) F8s {
   float4 a, b;
 };
@@ -62,17 +59,12 @@ PT_RECON_FN void reconstruct_hit(const DevScene& sc, int prim, float b0, float b
   const V3 p0 = mk3(v0), p1 = mk3(v1), p2 = mk3(v2);
   const uint32_t flags = __float_as_uint(v2.w) & 0xffu;
   V2 uv[3];
-#if PT_PACKED_SHADING
   // the triangle's shading attributes come from its own 64-byte record (dev_scene.cuh tri_shade): two 32-byte loads that
   // depend on the primitive id only, instead of the index triple and up to fifteen gathers behind it
   const F8s sb = ld256_nc(reinterpret_cast<const F8s*>(sc.tri_shade + 4 * (size_t)prim) + 1);
   uv[0] = V2{sb.a.y, sb.a.z};
   uv[1] = V2{sb.a.w, sb.b.x};
   uv[2] = V2{sb.b.y, sb.b.z};
-#else
-  const uint4 idx = __ldg(sc.tri_index + prim);
-  tri_uvs(sc, idx, flags, uv);
-#endif
   V3 dpdu, dpdv;
   tri_partials(p0, p1, p2, uv, &dpdu, &dpdv);
   float x_abs_sum = fabsf(b0 * p0.x) + fabsf(b1 * p1.x) + fabsf(b2 * p2.x);
@@ -95,12 +87,8 @@ PT_RECON_FN void reconstruct_hit(const DevScene& sc, int prim, float b0, float b
   if (has_n || has_s) {
     V3 ns;
     if (has_n) {
-#if PT_PACKED_SHADING
       const F8s sa = ld256_nc(reinterpret_cast<const F8s*>(sc.tri_shade + 4 * (size_t)prim));  // same 64-byte line as sb
       ns = b0 * mk3(sa.a.x, sa.a.y, sa.a.z) + b1 * mk3(sa.a.w, sa.b.x, sa.b.y) + b2 * mk3(sa.b.z, sa.b.w, sb.a.x);
-#else
-      ns = b0 * load3(sc.normal, idx.x) + b1 * load3(sc.normal, idx.y) + b2 * load3(sc.normal, idx.z);
-#endif
       if (norm_squared(ns) > 0.0f) ns = normalize(ns);
       else ns = si->g.n;
     } else {
@@ -108,9 +96,7 @@ PT_RECON_FN void reconstruct_hit(const DevScene& sc, int prim, float b0, float b
     }
     V3 ss;
     if (has_s) {
-#if PT_PACKED_SHADING
       const uint4 idx = __ldg(sc.tri_index + prim);  // tangents (glTF only) stay per vertex
-#endif
       ss = b0 * load3(sc.tangent, idx.x) + b1 * load3(sc.tangent, idx.y) + b2 * load3(sc.tangent, idx.z);
       if (norm_squared(ss) > 0.0f) ss = normalize(ss);
       else ss = normalize(dpdu);

@@ -166,9 +166,7 @@ __global__ void __launch_bounds__(256) radix_tree_kernel(const uint64_t* __restr
   }
 }
 
-#ifndef PT_BVH_MAX_LEAF
 #define PT_BVH_MAX_LEAF 4u  // BVH::new(.., &4), importer/mitsuba.rs:362
-#endif
 
 __device__ __forceinline__ float box_area(float4 mn, float4 mx) {
   const float dx = mx.x - mn.x, dy = mx.y - mn.y, dz = mx.z - mn.z;
@@ -233,9 +231,7 @@ __global__ void __launch_bounds__(256) refit_kernel(uint32_t n, BuildArrays A) {
 // decision (same criterion as refit_kernel) and the interior-node counts are known at merge time, so there is no
 // separate refit pass.  Merged clusters are not contiguous ranges of the sorted order, so the primitives' final order
 // is the depth-first order of the finished tree (ploc_positions_kernel).
-#ifndef PLOC_R
 #define PLOC_R 16
-#endif
 #define PLOC_BLOCK 256
 #define PLOC_NONE 0xffffffffu
 #define PLOC_MAX_ROUNDS 512

@@ -106,9 +106,7 @@ __global__ void __launch_bounds__(128) shade_miss_kernel(const __grid_constant__
 // segment, integrator.rs:66-80) + Ld_bsdf (emitted radiance found by the MIS ray, integrator.rs:113-135), then
 // L += beta * n_lights * Ld (integrator.rs:443-447, uniform_sample_one_light :216).  One thread per record =
 // one writer per path, so the per-path summation order is the reference's.
-#ifndef PT_RESOLVE_MIN_BLOCKS
 #define PT_RESOLVE_MIN_BLOCKS 4  // 64 registers, no spills: 32 warps per SM for what is a streaming pass with a rare heavy branch
-#endif
 __global__ void __launch_bounds__(256, PT_RESOLVE_MIN_BLOCKS) connect_resolve_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ PathArrays P, const int* __restrict__ q_nee, RoundCounters* ctr) {
   const uint32_t n = ctr->n_nee;
   const uint32_t stride = gridDim.x * blockDim.x;

@@ -64,15 +64,7 @@ PT_DEV void nee_prepare(const DevScene& sc, const SurfInter& si, const Bsdf& bsd
   *nee_flags = nf;
 }
 
-#ifndef PT_SHADE_PARAM
-#define PT_SHADE_PARAM  // by value: with __grid_constant__ the 128-register shade kernels spill more (measured slower)
-#endif
-#ifndef PT_SHADE_MIN_BLOCKS
 #define PT_SHADE_MIN_BLOCKS 4
-#endif
-#ifndef PT_SHADE_BLOCK
-#define PT_SHADE_BLOCK 128
-#endif
 
 // EXACT only names the build: the exact instantiation comes from a translation unit compiled with IEEE division /
 // square root and without FMA contraction (PtrsRenderParams.flags & PTRS_RENDER_EXACT_SHADING, Makefile EXACTSHADE),
@@ -80,8 +72,9 @@ PT_DEV void nee_prepare(const DevScene& sc, const SurfInter& si, const Bsdf& bsd
 #ifndef PT_SHADE_EXACT
 #define PT_SHADE_EXACT 0
 #endif
+// sc and P by value: with __grid_constant__ the 128-register shade kernels spill more (measured slower)
 template <int MAT, bool EXACT>
-__global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_kernel(const __grid_constant__ RenderConst rc, PT_SHADE_PARAM DevScene sc, PT_SHADE_PARAM PathArrays P,
+__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) shade_kernel(const __grid_constant__ RenderConst rc, DevScene sc, PathArrays P,
                                                      const int* __restrict__ q, const float4* __restrict__ q_hit, int* __restrict__ q_ext_next,
                                                      int* __restrict__ q_nee, RoundCounters* ctr, RoundCounters* ctr_next) {
   const uint32_t n = ctr->n_class[MAT];
@@ -119,11 +112,7 @@ __global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_ker
         prefetch_l1(&P.slot[p_next]);
         prefetch_l1(sc.tri_verts + 3 * (size_t)prim_next);
         prefetch_l1(sc.tri_verts + 3 * (size_t)prim_next + 2);
-#if PT_PACKED_SHADING
         prefetch_l1(sc.tri_shade + 4 * (size_t)prim_next);
-#else
-        prefetch_l1(sc.tri_index + prim_next);
-#endif
       }
       uint32_t flags = pr.packed & 0x00ffffffu;
       int bounces = packed_bounces(pr.packed);
@@ -297,7 +286,7 @@ __global__ void __launch_bounds__(PT_SHADE_BLOCK, PT_SHADE_MIN_BLOCKS) shade_ker
 #endif
 void PT_SHADE_LAUNCHER(cudaStream_t st, int sm, const RenderConst& rc, const DevScene& sc, const PathArrays& P, const int* q,
                                          const float4* q_hit, int* q_next, int* q_nee, RoundCounters* ctr, RoundCounters* ctr_next) {
-  shade_kernel<PT_SHADE_MAT, PT_SHADE_EXACT != 0><<<PT_GRID((shade_kernel<PT_SHADE_MAT, PT_SHADE_EXACT != 0>), PT_SHADE_BLOCK, sm), PT_SHADE_BLOCK, 0, st>>>(rc, sc, P, q, q_hit, q_next, q_nee, ctr, ctr_next);
+  shade_kernel<PT_SHADE_MAT, PT_SHADE_EXACT != 0><<<PT_GRID((shade_kernel<PT_SHADE_MAT, PT_SHADE_EXACT != 0>), 128, sm), 128, 0, st>>>(rc, sc, P, q, q_hit, q_next, q_nee, ctr, ctr_next);
 }
 
 }  // namespace ptrs

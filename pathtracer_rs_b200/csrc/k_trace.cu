@@ -2,9 +2,7 @@
 #include "launch.hpp"
 #include "wavefront.cuh"
 
-#ifndef PT_TRACE_MIN_BLOCKS
 #define PT_TRACE_MIN_BLOCKS 8
-#endif
 
 namespace ptrs {
 

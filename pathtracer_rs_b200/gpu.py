@@ -19,7 +19,7 @@ from ._abi import *  # noqa: F401,F403
 from .host import HIT_DTYPE, RAY_DTYPE, FlatScene, default_render_params
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("PTRS_B200_LIB") or os.path.join(_HERE, "lib", "libptrs_b200.so")  # override = tuning variants only
+LIB_PATH = os.environ.get("PTRS_B200_LIB") or os.path.join(_HERE, "lib", "libptrs_b200.so")  # override: A/B another build of the library
 _LIB = None
 
 EXPORTS = [
