@@ -23,7 +23,7 @@ BLOB := $(abspath pathtracer_rs_b200/data/sobol_tables.bin)
 
 DEV_HDRS  := $(wildcard $(CS)/*.cuh) $(CS)/launch.hpp $(CS)/handles.hpp include/ptrs_b200.h
 SHADE_OBJ := $(foreach m,0 1 2 3 4 5,$(OBJ)/k_shade_$(m).o $(OBJ)/k_shade_exact_$(m).o)
-CUDA_OBJ  := $(OBJ)/ptrs_b200.o $(OBJ)/multi_gpu.o $(OBJ)/k_probe_fast.o $(OBJ)/k_probe_exact.o $(OBJ)/k_trace.o $(OBJ)/k_misc.o $(OBJ)/k_bvh.o $(OBJ)/k_tables.o $(SHADE_OBJ) $(OBJ)/sobol_blob.o
+CUDA_OBJ  := $(OBJ)/ptrs_b200.o $(OBJ)/multi_gpu.o $(OBJ)/k_probe_fast.o $(OBJ)/k_probe_exact.o $(OBJ)/k_trace.o $(OBJ)/k_misc.o $(OBJ)/k_bvh.o $(OBJ)/k_sah.o $(OBJ)/k_tables.o $(SHADE_OBJ) $(OBJ)/sobol_blob.o
 
 all: $(LIB)/libptrs_b200.so $(LIB)/libptrs_host.so oracle/_build/liboracle.so examples
 

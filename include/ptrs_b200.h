@@ -328,7 +328,14 @@ int32_t ptrs_scene_create(const PtrsSceneDesc* desc, PtrsScene** out);
  * traversal cost and the winner among hits within an ulp of each other can differ (the reference's traversal
  * resolves those by visit order). */
 int32_t ptrs_scene_create_device_bvh(const PtrsSceneDesc* desc, PtrsScene** out);
-/* node count of the device-side tree (either constructor) and the device build time (0 for a host-built BVH) */
+/* Same, but the accelerator is the reference's own: BVH::new(prims, max_prims_in_node) (accelerator.rs:103-346) built
+ * on the device.  The tree equals the one BVH::new builds over the primitives in the order given, record for record
+ * and in its primitive order, so hits (prim, t, barycentrics), traversal counters and any-hit answers equal those of
+ * ptrs_scene_create over that tree, bit for bit.  desc->nodes / n_nodes are ignored; PtrsLight.prim and the prim ids
+ * reported by ptrs_intersect* refer to the caller's order.  max_prims_in_node: 1 .. 65535 (the importers use 4).
+ * A tree deeper than the 64-entry traversal stack is refused with PTRS_ERR_UNSUPPORTED, as by ptrs_scene_create. */
+int32_t ptrs_scene_create_sah_bvh(const PtrsSceneDesc* desc, int32_t max_prims_in_node, PtrsScene** out);
+/* node count of the device-side tree (any constructor) and the device build time (0 for a host-built BVH) */
 int32_t ptrs_scene_bvh_info(const PtrsScene* scene, uint32_t* n_nodes, float* device_build_ms);
 /* The device-side tree for inspection: 32-byte LinearBVHNode records in the traversal layout (root in slot 0, slot 1
  * unused, the two children of an interior node at offset and offset + 1); prim_order (optional, device-built trees

@@ -63,6 +63,10 @@ int validate_prims_on_device(cudaStream_t st, uint32_t n, const uint32_t* prim_v
 int pair_layout_on_device(cudaStream_t st, const float4* d_raw, uint32_t n, uint32_t n_interior, float4** out, uint32_t* n_out);
 void launch_remap_light_prims(cudaStream_t st, PtrsLight* lights, uint32_t n_lights, const uint32_t* inv_perm);
 
+// k_sah.cu: the reference's SAH tree (ptrs_host::build_bvh) built on the device, bit for bit
+int build_sah_bvh_on_device(cudaStream_t st, uint32_t n, const uint32_t* d_prim_vertex, const float* d_pos, int max_prims, uint32_t depth_limit,
+                            float4** nodes_out, uint32_t* n_nodes_out, uint32_t** perm_out, uint32_t* max_depth_out);
+
 // k_probe.cu, built twice (shade-kernel arithmetic / exact arithmetic)
 #define PT_DECL_PROBES(SUF)                                                                                                                       \
   void launch_bxdf_eval_probe_##SUF(cudaStream_t st, const PtrsLobeDesc& d, const float* wo, const float* wi, uint32_t n, float* out);             \

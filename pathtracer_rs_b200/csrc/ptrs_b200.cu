@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -610,8 +611,13 @@ static bool build_occlusion_tree(const PtrsBvhNode* nodes, uint32_t n_nodes, std
   return true;
 }
 
-static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsScene** out) {
+// where a scene's tree comes from: the caller's records (ptrs_scene_create), the library's PLOC build
+// (ptrs_scene_create_device_bvh) or the reference's SAH build on the device (ptrs_scene_create_sah_bvh)
+enum class TreeSource { kCaller, kPloc, kSah };
+
+static int32_t scene_create_impl(const PtrsSceneDesc* d, TreeSource tree, int32_t max_prims_in_node, PtrsScene** out) {
   if (!d || !out) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+  const bool device_bvh = tree != TreeSource::kCaller;
   if (d->abi_version != PTRS_ABI_VERSION) return fail(PTRS_ERR_INVALID_ARGUMENT, "PtrsSceneDesc.abi_version mismatch");
   if (d->n_prims > 0 && ((!device_bvh && !d->nodes) || !d->prim_vertex || !d->prim_mesh || !d->prim_material || !d->prim_area_light || !d->pos || !d->meshes))
     return fail(PTRS_ERR_INVALID_ARGUMENT, "missing geometry arrays");
@@ -731,7 +737,7 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
     if (bad & 4) return fail(PTRS_ERR_INVALID_ARGUMENT, "prim_area_light names a light that is not an area light");
     CUDA_TRY(s->tri_verts.alloc((size_t)d->n_prims * 3));
     CUDA_TRY(s->tri_index.alloc(d->n_prims));
-    if (device_bvh) {
+    if (tree == TreeSource::kPloc) {
       // unordered primitives in, BVH built and triangles laid out on the device (k_bvh.cu)
       CUDA_TRY(inv.alloc(d->n_prims));
       cudaEvent_t e0, e1;
@@ -770,6 +776,55 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
         s->world_bound[4] = root[4];
         s->world_bound[5] = root[5];
       }
+    } else if (tree == TreeSource::kSah) {
+      // the reference's tree over the caller's primitive order, built on the device (k_sah.cu); from its records on the
+      // scene is assembled as ptrs_scene_create assembles the same records
+      CUDA_TRY(inv.alloc(d->n_prims));
+      cudaEvent_t e0, e1;
+      CUDA_TRY(cudaEventCreate(&e0));
+      CUDA_TRY(cudaEventCreate(&e1));
+      CUDA_TRY(cudaEventRecord(e0, 0));
+      DevBuf<float4> raw;
+      uint32_t n_raw = 0, max_depth = 0, *perm = nullptr;
+      const int be = build_sah_bvh_on_device(0, d->n_prims, pv.p, pos.p, max_prims_in_node, PT_STACK_SIZE + 1, &raw.p, &n_raw, &perm, &max_depth);
+      if (be != (int)cudaSuccess) return fail(PTRS_ERR_CUDA, std::string("device SAH build: ") + cudaGetErrorString((cudaError_t)be));
+      raw.n = (size_t)n_raw * 2;
+      s->prim_map.p = perm;
+      s->prim_map.n = d->n_prims;
+      // the depth rule of the caller's trees above: the builder's max_depth counts the deepest leaf, a traversal's stack holds
+      // one entry per interior level
+      if (max_depth > PT_STACK_SIZE + 1) return fail(PTRS_ERR_UNSUPPORTED, "BVH deeper than the 64-entry traversal stack (accelerator.rs:366)");
+      s->bvh_depth = max_depth - 1;
+      float4* nodes = nullptr;
+      const int pe = pair_layout_on_device(0, raw.p, n_raw, (n_raw - 1) / 2, &nodes, &n_dev_nodes);
+      if (pe != (int)cudaSuccess) return fail(PTRS_ERR_CUDA, std::string("BVH re-layout: ") + cudaGetErrorString((cudaError_t)pe));
+      s->nodes.p = nodes;
+      s->nodes.n = (size_t)n_dev_nodes * 2;
+      launch_assemble_tris(0, d->n_prims, perm, pv.p, pos.p, pm.p, pmat.p, pal.p, s->meshes.p, s->tri_verts.p, s->tri_index.p, inv.p);
+      launch_remap_light_prims(0, s->lights.p, d->n_lights, inv.p);
+      CUDA_TRY(cudaEventRecord(e1, 0));
+      CUDA_TRY(cudaEventSynchronize(e1));
+      CUDA_TRY(cudaGetLastError());
+      cudaEventElapsedTime(&s->bvh_build_ms, e0, e1);
+      cudaEventDestroy(e0);
+      cudaEventDestroy(e1);
+      s->scene_bytes += (uint64_t)n_dev_nodes * 32 + (uint64_t)d->n_prims * 4;
+      // the occlusion tree: the host collapse of ptrs_scene_create, over the records copied back
+      const auto t0 = std::chrono::steady_clock::now();
+      std::vector<PtrsBvhNode> recs(n_raw);
+      CUDA_TRY(cudaMemcpyAsync(recs.data(), raw.p, (size_t)n_raw * 32, cudaMemcpyDeviceToHost, 0));
+      CUDA_TRY(cudaStreamSynchronize(0));
+      std::memcpy(s->world_bound, recs[0].bounds_min, 12);
+      std::memcpy(s->world_bound + 3, recs[0].bounds_max, 12);
+      std::vector<float4> wide;
+      if (build_occlusion_tree(recs.data(), n_raw, &wide)) {
+        CUDA_TRY(s->wnodes.upload(wide.data(), wide.size()));
+        s->scene_bytes += (uint64_t)wide.size() * 16;
+      }
+      if (std::getenv("PTRS_BVH_DEBUG"))
+        std::fprintf(stderr, "sah build: occlusion tree (copy-back + host collapse) %9.3f ms\n",
+                     std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
+      CUDA_TRY(cudaStreamSynchronize(0));  // the staging buffers above are released when this scope ends
     } else {
       // reference-built tree: the 32 B records are kept, but the two children of every interior node are placed side
       // by side (64 B pairs in depth-first order, root alone in slot 0) so that one traversal step reads one
@@ -979,8 +1034,8 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
   v.pop_twice = n_dev_nodes > 4096u ? 1u : 0u;
   if (const char* e = std::getenv("PTRS_POP_TWICE")) v.pop_twice = std::atoi(e) != 0;  // tuning only
   // a reference-built tree is walked in the reference's order (dir_is_neg[axis]); a tree built here front to back
-  v.dist_order = device_bvh ? 1u : 0u;
-  if (const char* e = std::getenv("PTRS_DIST_ORDER")) v.dist_order = device_bvh && std::atoi(e) != 0;  // tuning only
+  v.dist_order = tree == TreeSource::kPloc ? 1u : 0u;
+  if (const char* e = std::getenv("PTRS_DIST_ORDER")) v.dist_order = tree == TreeSource::kPloc && std::atoi(e) != 0;  // tuning only
   if (const char* e = std::getenv("PTRS_BOX_MIN")) v.box_min = (uint32_t)std::max(1, std::min(32, std::atoi(e)));  // tuning only
   v.wnodes = s->wnodes.p;
   v.n_wnodes = d->n_prims > 0 ? (uint32_t)(s->wnodes.n / 8) : 0u;
@@ -1007,8 +1062,13 @@ static int32_t scene_create_impl(const PtrsSceneDesc* d, bool device_bvh, PtrsSc
   return PTRS_OK;
 }
 
-int32_t ptrs_scene_create(const PtrsSceneDesc* d, PtrsScene** out) { return scene_create_impl(d, false, out); }
-int32_t ptrs_scene_create_device_bvh(const PtrsSceneDesc* d, PtrsScene** out) { return scene_create_impl(d, true, out); }
+int32_t ptrs_scene_create(const PtrsSceneDesc* d, PtrsScene** out) { return scene_create_impl(d, TreeSource::kCaller, 0, out); }
+int32_t ptrs_scene_create_device_bvh(const PtrsSceneDesc* d, PtrsScene** out) { return scene_create_impl(d, TreeSource::kPloc, 0, out); }
+int32_t ptrs_scene_create_sah_bvh(const PtrsSceneDesc* d, int32_t max_prims_in_node, PtrsScene** out) {
+  // LinearBVHNode counts a leaf's primitives in 16 bits (accelerator.rs:89-95)
+  if (max_prims_in_node < 1 || max_prims_in_node > 65535) return fail(PTRS_ERR_INVALID_ARGUMENT, "max_prims_in_node must be in 1..65535");
+  return scene_create_impl(d, TreeSource::kSah, max_prims_in_node, out);
+}
 
 int32_t ptrs_scene_bvh_info(const PtrsScene* scene, uint32_t* n_nodes, float* device_build_ms) {
   if (!scene) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");

@@ -33,6 +33,7 @@ EXPORTS = [
     "ptrs_multi_create", "ptrs_multi_destroy", "ptrs_multi_device_count", "ptrs_multi_render", "ptrs_multi_root_film", "ptrs_multi_scene",
     "ptrs_comm_unique_id", "ptrs_comm_init_rank", "ptrs_comm_destroy", "ptrs_comm_info", "ptrs_film_reduce",
     "ptrs_bxdf_eval", "ptrs_bxdf_sample", "ptrs_light_sample", "ptrs_light_pdf", "ptrs_scene_download_mipmaps", "ptrs_scene_download_env",
+    "ptrs_scene_create_sah_bvh",
 ]
 
 
@@ -58,6 +59,7 @@ def lib():
         L.ptrs_set_device.argtypes = [i32]
         L.ptrs_scene_create.argtypes = [descp, C.POINTER(vp)]
         L.ptrs_scene_create_device_bvh.argtypes = [descp, C.POINTER(vp)]
+        L.ptrs_scene_create_sah_bvh.argtypes = [descp, i32, C.POINTER(vp)]
         L.ptrs_scene_bvh_info.argtypes = [vp, C.POINTER(C.c_uint32), fp]
         L.ptrs_scene_download_nodes.argtypes = [vp, C.POINTER(PtrsBvhNode), C.c_uint32, C.POINTER(C.c_uint32)]
         L.ptrs_scene_destroy.argtypes = [vp]
@@ -199,16 +201,23 @@ class Film:
 class RenderScene:
     """Device copy of a flattened scene (src/pathtracer/mod.rs:84-106)."""
 
-    def __init__(self, flat, device_bvh=False, device_tables=False):
+    def __init__(self, flat, device_bvh=False, device_tables=False, sah_on_device=False, max_prims_in_node=4):
         """device_bvh=True ignores the description's nodes and builds the tree on the GPU (ptrs_scene_create_device_bvh: Morton order + PLOC);
+        sah_on_device=True ignores them too and builds the reference's SAH tree over the description's primitive order on the GPU
+        (ptrs_scene_create_sah_bvh, leaves of at most max_prims_in_node primitives);
         device_tables=True hands over level 0 of every MIP pyramid only and no env Distribution2D: the library builds them."""
+        if device_bvh and sah_on_device:
+            raise ValueError("device_bvh and sah_on_device select different trees")
         desc = (flat.desc_device_tables if device_tables else flat.desc) if isinstance(flat, FlatScene) else flat
         h = C.c_void_p()
-        _check((lib().ptrs_scene_create_device_bvh if device_bvh else lib().ptrs_scene_create)(desc, C.byref(h)))
+        if sah_on_device:
+            _check(lib().ptrs_scene_create_sah_bvh(desc, max_prims_in_node, C.byref(h)))
+        else:
+            _check((lib().ptrs_scene_create_device_bvh if device_bvh else lib().ptrs_scene_create)(desc, C.byref(h)))
         self._h = h
         self.n_lights = desc.contents.n_lights
         self.n_prims = desc.contents.n_prims
-        self.device_bvh = device_bvh
+        self.device_bvh = device_bvh or sah_on_device  # the scene keeps a primitive order of its own
 
     def bvh_info(self):
         """(device node count, device build time in ms; 0 for a host-built tree)"""
