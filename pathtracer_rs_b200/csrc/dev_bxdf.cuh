@@ -50,7 +50,7 @@ PT_DEV V2 concentric_sample_disk(V2 u) {  // sampling.rs:96-116
     r = oy;
     theta = PT_FRAC_PI_2 - PT_FRAC_PI_4 * (ox / oy);
   }
-  return V2{r * cosf(theta), r * sinf(theta)};
+  return V2{r * cos_small_angle(theta), r * sin_small_angle(theta)};
 }
 PT_DEV V3 cosine_sample_hemisphere(V2 u) {  // sampling.rs:118-122
   V2 d = concentric_sample_disk(u);
@@ -198,8 +198,8 @@ PT_DEV void trowbridge_reitz_sample_11(float cos_t, float u1, float u2, float* s
   if (cos_t > 0.9999f) {
     float r = sqrtf(u1 / (1.f - u1));
     float phi = 6.28318530718f * u2;
-    *slope_x = r * cosf(phi);
-    *slope_y = r * sinf(phi);
+    *slope_x = r * cos_small_angle(phi);
+    *slope_y = r * sin_small_angle(phi);
     return;
   }
   float sin_t = sqrtf(fmaxf(0.0f, 1.f - cos_t * cos_t));
@@ -457,7 +457,9 @@ PT_DEV Spec bsdf_sample_f(const Bsdf& b, V3 wo_w, V3* wi_w, V2 u, float* pdf, ui
       }
       count -= 1;
     }
-  const Lobe& lobe = b.lobes[sel];
+  // A material with one lobe kind has at most one lobe, so sel == 0: b.lobes indexed with the run-time `sel` would keep
+  // the whole BSDF in local memory.  Disney's two lobes keep the indexed access.
+  const Lobe& lobe = pt_popc(PT_LOBE_MASK) == 1 ? b.lobes[0] : b.lobes[sel];
   V2 u_remapped{(u.x * (float)matching) - (float)comp, u.y};
   V3 wi = mk3(0, 0, 0);
   V3 wo = world_to_local(b, wo_w);

@@ -126,6 +126,21 @@ PT_DEV int abs_mod(int a, int b) {  // math.rs:237-244
   int r = a - (a / b) * b;
   return r < 0 ? r + b : r;
 }
+// sinf / cosf of an angle below 105615 radians in magnitude, the range on which libdevice reduces the argument with three
+// multiply-adds: its large-argument branch (Payne-Hanek, with a 28-byte local array) is compiled out, so the shade
+// kernels that call these keep no local-memory frame.  Same values as sinf / cosf on that range, NaN included.
+// PRECONDITION: |x| < 105615 or x is NaN.  A larger or infinite argument is undefined behaviour, not a wrong value; use
+// sinf / cosf for any angle that is not bounded by construction.  The callers (concentric disk, GGX phi, environment
+// sample, acos-based theta) all pass angles within [-2 pi, 2 pi]: a Sobol or table sample in [0, 1] scaled by at most
+// 2 pi, or an acos.
+PT_DEV float sin_small_angle(float x) {
+  if (fabsf(x) >= 105615.0f) __builtin_unreachable();
+  return sinf(x);
+}
+PT_DEV float cos_small_angle(float x) {
+  if (fabsf(x) >= 105615.0f) __builtin_unreachable();
+  return cosf(x);
+}
 PT_DEV float lerpf(float x, float y, float a) { return x * (1.0f - a) + y * a; }  // math.rs:250
 PT_DEV uint64_t cantor_pairing(uint64_t x, uint64_t y) { return (x + y) * (x + y + 1) / 2 + y; }  // math.rs:256
 

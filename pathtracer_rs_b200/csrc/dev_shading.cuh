@@ -122,7 +122,7 @@ PT_RECON_FN void reconstruct_hit(const DevScene& sc, int prim, float b0, float b
 struct RayDiff {
   V3 rx_o, ry_o, rx_d, ry_d;
 };
-PT_DEVN void compute_differentials(SurfInter* si, const RayDiff& rd) {
+PT_DEV void compute_differentials(SurfInter* si, const RayDiff& rd) {
   const V3 n = si->g.n, p = si->g.p;
   float d = dot(n, p);
   float tx = -(dot(n, rd.rx_o) - d) / dot(n, rd.rx_d);
@@ -151,11 +151,10 @@ PT_DEVN void compute_differentials(SurfInter* si, const RayDiff& rd) {
 
 PT_DEV TexCoord tc_of(const SurfInter& si) { return TexCoord{si.uv.x, si.uv.y, si.dudx, si.dvdx, si.dudy, si.dvdy}; }
 
-PT_DEVN void normal_mapping(const DevScene& sc, int tex, SurfInter* si) {  // material/mod.rs:39-79
+PT_DEV void normal_mapping(const DevScene& sc, int tex, SurfInter* si) {  // material/mod.rs:39-79
   const V3 c0 = si->sh_dpdu, c1 = si->sh_dpdv, c2 = si->sh_n;
-  float o[3];
-  tex_eval(sc, tex, tc_of(*si), o);
-  V3 tn = normalize(mk3(o[0], o[1], o[2]));
+  const Spec o = tex_eval(sc, tex, tc_of(*si));
+  V3 tn = normalize(mk3(o.r, o.g, o.b));
   V3 ns = normalize(mk3(c0.x * tn.x + c1.x * tn.y + c2.x * tn.z, c0.y * tn.x + c1.y * tn.y + c2.y * tn.z, c0.z * tn.x + c1.z * tn.y + c2.z * tn.z));
   V3 ss = si->sh_dpdu;
   V3 ts = cross(ss, ns);
@@ -330,7 +329,7 @@ PT_DEV float dist1d_sample(const float* func, const float* cdf, float func_int, 
   *pdf = func_int > 0.0f ? __ldg(func + offset) / func_int : 0.0f;
   return ((float)offset + du) / (float)n;
 }
-PT_DEVN V2 dist2d_sample(const DevEnv& e, V2 u, float* pdf) {  // sampling.rs:211-221
+PT_DEV V2 dist2d_sample(const DevEnv& e, V2 u, float* pdf) {  // sampling.rs:211-221
   float p0, p1;
   size_t v, dummy;
   float d1 = dist1d_sample(e.marg_func, e.marg_cdf, e.marg_func_int, e.nv, u.y, &p1, &v, e.marg_guide, e.kv);
@@ -345,11 +344,7 @@ PT_DEV float dist2d_pdf(const DevEnv& e, float px, float py) {  // sampling.rs:2
   if (iv > (unsigned long long)e.nv - 1) iv = e.nv - 1;
   return __ldg(e.cond_func + iv * e.nu + iu) / e.marg_func_int;
 }
-PT_DEV Spec env_lookup(const DevScene& sc, const DevEnv& e, float s, float t) {
-  float o[3];
-  mip_lookup_width(sc, sc.mipmaps[e.mip], s, t, 0.0f, o);
-  return sp(o[0], o[1], o[2]);
-}
+PT_DEV Spec env_lookup(const DevScene& sc, const DevEnv& e, float s, float t) { return mip_lookup_width(sc, sc.mipmaps[e.mip], s, t, 0.0f); }
 // InfiniteAreaLight::le, light.rs:488-498
 PT_DEV Spec env_le(const DevScene& sc, const PtrsLight& l, V3 ray_d) {
   const DevEnv& e = sc.envs[l.env];
@@ -392,7 +387,7 @@ PT_DEVN TriPoint triangle_sample(const DevScene& sc, int prim, V2 u) {  // shape
 }
 
 // Triangle::pdf_at_point, shape.rs:62-72: a single-triangle Triangle::intersect from `ref` along wi
-PT_DEVN float triangle_pdf_at_point(const DevScene& sc, int prim, const Inter& ref, V3 wi, float area) {
+PT_DEVN float triangle_pdf_at_point(const DevScene& sc, int prim, Inter ref, V3 wi, float area) {
   V3 o;
   spawn_ray(ref, wi, &o);
   const float4 v0 = __ldg(sc.tri_verts + 3 * (size_t)prim), v1 = __ldg(sc.tri_verts + 3 * (size_t)prim + 1),
@@ -453,8 +448,8 @@ PT_DEV void light_sample_li(const DevScene& sc, const PtrsLight& light, const In
     V2 uv = dist2d_sample(e, u, &map_pdf);
     if (map_pdf != 0.0f) {
       float theta = uv.y * PT_PI, phi = uv.x * 2.0f * PT_PI;
-      float cos_t = cosf(theta), sin_t = sinf(theta);
-      float sin_p = sinf(phi), cos_p = cosf(phi);
+      float cos_t = cos_small_angle(theta), sin_t = sin_small_angle(theta);
+      float sin_p = sin_small_angle(phi), cos_p = cos_small_angle(phi);
       out->wi = xform_vec(e.light_to_world, mk3(sin_t * cos_p, sin_t * sin_p, cos_t));
       out->pdf = sin_t == 0.0f ? 0.0f : map_pdf / (2.0f * PT_PI * PT_PI * sin_t);
       out->p1.p = ref.p + out->wi * (2.0f * light.world_radius);
@@ -469,7 +464,7 @@ PT_DEV float light_pdf_li(const DevScene& sc, const PtrsLight& light, const Inte
   const DevEnv& e = sc.envs[light.env];
   V3 wl = xform_vec(e.world_to_light, w);
   float theta = spherical_theta(wl), phi = spherical_phi(wl);
-  float sin_t = sinf(theta);
+  float sin_t = sin_small_angle(theta);
   return sin_t == 0.0f ? 0.0f : dist2d_pdf(e, phi * PT_INV_2_PI, theta * PT_FRAC_1_PI) / (2.0f * PT_PI * PT_PI * sin_t);
 }
 

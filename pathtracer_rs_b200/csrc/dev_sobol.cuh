@@ -104,9 +104,11 @@ PT_DEV void sampler_start(const SobolConfig& c, const SobolSplit& sp, PathSample
 }
 
 // generic path (sobol.rs:169-193): only reached for dimensions beyond the split tables
-PT_DEVN float sample_dimension_generic(const SobolConfig& c, const uint32_t* __restrict__ matrices, const PathSampler& s, uint32_t dim) {
-  const uint64_t index = sobol_interval_to_index(c, (uint64_t)s.sample, s.px - c.bounds_min[0], s.py - c.bounds_min[1]);
-  return sobol_sample(matrices, index, dim, s.scramble);
+// (the sampler's fields by value: a reference would keep the caller's PathSampler in local memory)
+PT_DEVN float sample_dimension_generic(const SobolConfig& c, const uint32_t* __restrict__ matrices, uint32_t sample, int32_t px, int32_t py,
+                                       uint32_t scramble, uint32_t dim) {
+  const uint64_t index = sobol_interval_to_index(c, (uint64_t)sample, px - c.bounds_min[0], py - c.bounds_min[1]);
+  return sobol_sample(matrices, index, dim, scramble);
 }
 
 PT_DEV float sample_dimension(const SobolConfig& c, const SobolSplit& sp, const uint32_t* __restrict__ matrices, const PathSampler& s, uint32_t dim) {
@@ -115,7 +117,7 @@ PT_DEV float sample_dimension(const SobolConfig& c, const SobolSplit& sp, const 
     const uint32_t raw = __ldg(sp.tab + s.row_s + dim) ^ __ldg(sp.tab + s.row_x + dim) ^ __ldg(sp.tab + s.row_y + dim) ^ s.scramble;
     v = fminf(PT_ONE_MINUS_EPSILON, (float)raw * 0x1.p-32f);
   } else {
-    v = sample_dimension_generic(c, matrices, s, dim);
+    v = sample_dimension_generic(c, matrices, s.sample, s.px, s.py, s.scramble, dim);
   }
   if (dim == 0 || dim == 1) {
     int32_t pmin = dim == 0 ? c.bounds_min[0] : c.bounds_min[1];

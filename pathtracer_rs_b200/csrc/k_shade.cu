@@ -72,9 +72,10 @@ PT_DEV void nee_prepare(const DevScene& sc, const SurfInter& si, const Bsdf& bsd
 #ifndef PT_SHADE_EXACT
 #define PT_SHADE_EXACT 0
 #endif
-// sc and P by value: with __grid_constant__ the 128-register shade kernels spill more (measured slower)
+// sc as __grid_constant__: the area-light helpers that stay calls (triangle_sample, triangle_pdf_at_point) take it by
+// reference, and a by-value parameter whose address is taken is copied into a local-memory frame.  P by value.
 template <int MAT, bool EXACT>
-__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) shade_kernel(const __grid_constant__ RenderConst rc, DevScene sc, PathArrays P,
+__global__ void __launch_bounds__(128, PT_SHADE_MIN_BLOCKS) shade_kernel(const __grid_constant__ RenderConst rc, const __grid_constant__ DevScene sc, PathArrays P,
                                                      const int* __restrict__ q, const float4* __restrict__ q_hit, int* __restrict__ q_ext_next,
                                                      int* __restrict__ q_nee, RoundCounters* ctr, RoundCounters* ctr_next) {
   const uint32_t n = ctr->n_class[MAT];

@@ -50,18 +50,16 @@ __global__ void __launch_bounds__(256) env_density_kernel(const __grid_constant_
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int u = (int)(i % (uint32_t)nu), v = (int)(i / (uint32_t)nu);
     const float up = ((float)u + 0.5f) / (float)nu, vp = ((float)v + 0.5f) / (float)nv;
-    float c[3] = {0.f, 0.f, 0.f};
+    Spec c;
     if (mode == 0) {
-      mip_triangle(sc, mm, 0, up, vp, c);
+      c = mip_triangle(sc, mm, 0, up, vp);
     } else if (mode == 1) {
-      mip_triangle(sc, mm, mm.n_levels - 1, up, vp, c);
+      c = mip_triangle(sc, mm, mm.n_levels - 1, up, vp);
     } else {
-      float a[3], b[3];
-      mip_triangle(sc, mm, il, up, vp, a);
-      mip_triangle(sc, mm, il + 1, up, vp, b);
-      for (int k = 0; k < 3; ++k) c[k] = a[k] * (1.0f - delta) + b[k] * delta;
+      const Spec a = mip_triangle(sc, mm, il, up, vp), b = mip_triangle(sc, mm, il + 1, up, vp);
+      c = sp(a.r * (1.0f - delta) + b.r * delta, a.g * (1.0f - delta) + b.g * delta, a.b * (1.0f - delta) + b.b * delta);
     }
-    const float y = c[0] * 0.212671f + c[1] * 0.715160f + c[2] * 0.072169f;  // spectrum.rs:112-115
+    const float y = c.r * 0.212671f + c.g * 0.715160f + c.b * 0.072169f;  // spectrum.rs:112-115
     func[i] = row_sin[v] * y;
   }
 }
