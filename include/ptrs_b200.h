@@ -386,11 +386,25 @@ int32_t ptrs_film_resolve_srgb8(PtrsFilm* film, uint8_t* rgba /* W*H*4 */); /* f
 float* ptrs_film_device_ptr(PtrsFilm* film);
 int32_t ptrs_film_sample_bounds(int32_t width, int32_t height, const float filter_radius[2],
                                 int32_t out_min_max[4]); /* film.rs:174-185 */
+/* The sample rectangle that completes a pixel crop: the smallest rectangle of sample positions ({x0, y0, x1, y1},
+ * half-open, in the coordinates of ptrs_film_sample_bounds) whose samples include every contribution any pixel of
+ * pixel_rect (half-open, inside the film) receives in a full render, clipped to the sample bounds.  Derived from the
+ * float expressions of the film splat; for radius 2 it is pixel_rect grown by 2 on each side.  Host arithmetic only. */
+int32_t ptrs_film_region_sample_rect(int32_t width, int32_t height, const float filter_radius[2], const int32_t pixel_rect[4],
+                                     int32_t sample_rect[4]);
 
 /* PathIntegrator */
 int32_t ptrs_render_params_default(PtrsRenderParams* params); /* integrator.rs:237-245 + Gaussian */
 int32_t ptrs_render(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params,
                     PtrsFilm* film, void* stream); /* integrator.rs:536; accumulates into film */
+/* ptrs_render restricted to a rectangle of sample positions: sample_rect = {x0, y0, x1, y1}, half-open, a non-empty
+ * rectangle inside ptrs_film_sample_bounds (so it may start at -2).  Every selected sample number (spp, sample range,
+ * stride / phase) of every position inside it is traced, with the same Sobol index as in the full render, and splatted
+ * into the full-size film; only film pixels within the filter footprint of the rectangle change.  Rectangles that
+ * partition the sample bounds sum to the full render (integrator.rs:545-637 renders 16x16 tiles of them).
+ * ptrs_stats counts camera_paths = area x selected samples.  ptrs_render is this call with the whole sample bounds. */
+int32_t ptrs_render_region(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params, const int32_t sample_rect[4],
+                           PtrsFilm* film, void* stream);
 /* li() of integrator.rs:579 for chosen (pixel, sample number) pairs: out_rgb[3 i ..] = radiance of that
  * camera path.  Same kernels as ptrs_render with the film splat left out; parity probe. */
 int32_t ptrs_path_radiance(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params,
@@ -422,6 +436,10 @@ int32_t ptrs_multi_device_count(const PtrsMultiScene* multi, int32_t* n_devices)
  * NULL) receives n_devices records; total_ms (may be NULL) the wall time of the whole call. */
 int32_t ptrs_multi_render(PtrsMultiScene* multi, const PtrsCamera* camera, const PtrsRenderParams* params,
                           float* host_rgbw, PtrsStats* per_device_stats, float* total_ms);
+/* the same restricted to a rectangle of sample positions, as ptrs_render_region; the reduce and the download still
+ * cover the whole film.  ptrs_multi_render is this call with the whole sample bounds. */
+int32_t ptrs_multi_render_region(PtrsMultiScene* multi, const PtrsCamera* camera, const PtrsRenderParams* params,
+                                 const int32_t sample_rect[4], float* host_rgbw, PtrsStats* per_device_stats, float* total_ms);
 /* the root film (owned by the handle; valid until the next ptrs_multi_render with another resolution) for
  * ptrs_film_resolve / ptrs_film_resolve_srgb8 */
 int32_t ptrs_multi_root_film(PtrsMultiScene* multi, PtrsFilm** film);

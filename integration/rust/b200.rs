@@ -256,6 +256,23 @@ pub fn render(
     rr_start_depth: i32,
     rr_enable: bool,
 ) {
+    render_region(log, gpu, camera, None, spp, max_depth, rr_threshold, rr_start_depth, rr_enable)
+}
+
+/// The same restricted to a rectangle of sample positions `[x0, y0, x1, y1]` (half-open, inside the film's sample
+/// bounds; `None` = all of them), e.g. one tile of integrator.rs:545-637 or, with `ptrs_film_region_sample_rect`, the
+/// samples that complete a pixel crop.  Only film pixels within the rectangle's filter footprint change.
+pub fn render_region(
+    log: &slog::Logger,
+    gpu: &B200Scene,
+    camera: &Camera,
+    sample_rect: Option<[i32; 4]>,
+    spp: usize,
+    max_depth: i32,
+    rr_threshold: f32,
+    rr_start_depth: i32,
+    rr_enable: bool,
+) {
     let mut params: ffi::PtrsRenderParams = unsafe { std::mem::zeroed() };
     unsafe { ffi::ptrs_render_params_default(&mut params) };
     params.spp = spp as i32; // rounded up to a power of two inside, like sobol.rs:37
@@ -267,7 +284,14 @@ pub fn render(
     let (w, h) = (cam.width, cam.height);
     let mut film = std::ptr::null_mut();
     let result = check(unsafe { ffi::ptrs_film_create(w, h, &mut film) })
-        .and_then(|_| check(unsafe { ffi::ptrs_render(gpu.handle, &cam, &params, film, std::ptr::null_mut()) }))
+        .and_then(|_| {
+            check(unsafe {
+                match sample_rect {
+                    Some(r) => ffi::ptrs_render_region(gpu.handle, &cam, &params, r.as_ptr(), film, std::ptr::null_mut()),
+                    None => ffi::ptrs_render(gpu.handle, &cam, &params, film, std::ptr::null_mut()),
+                }
+            })
+        })
         .and_then(|_| {
             let mut rgbw = vec![0f32; (w * h * 4) as usize];
             check(unsafe { ffi::ptrs_film_download(film, rgbw.as_mut_ptr()) }).map(|_| rgbw)

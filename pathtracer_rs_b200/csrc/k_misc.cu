@@ -7,17 +7,17 @@
 namespace ptrs {
 
 // ---- generate --------------------------------------------------------------------------------------
-// Work item w of a batch -> (sample j, pixel).  Pixels are enumerated in 8x4 blocks so that a warp
-// covers a compact screen tile (coherent primary rays); samples are the slow index.
+// Work item w of a batch -> (sample j, pixel).  Pixels of the enumerated rectangle are visited in 8x4 blocks
+// so that a warp covers a compact screen tile (coherent primary rays); samples are the slow index.
 PT_DEV void work_to_pixel(const RenderConst& rc, uint64_t w, int* px, int* py, int* sample) {
-  const uint32_t bw = ((uint32_t)rc.sb_ext[0] + 7u) >> 3, bh = ((uint32_t)rc.sb_ext[1] + 3u) >> 2;
+  const uint32_t bw = ((uint32_t)rc.rect_ext[0] + 7u) >> 3, bh = ((uint32_t)rc.rect_ext[1] + 3u) >> 2;
   const uint64_t per_sample = (uint64_t)bw * bh * 32u;
   const uint32_t j = (uint32_t)(w / per_sample);
   const uint32_t r = (uint32_t)(w % per_sample);
   const uint32_t blk = r >> 5, in = r & 31u;
   const uint32_t bx = blk % bw, by = blk / bw;
-  *px = rc.sb_min[0] + (int)(bx * 8u + (in & 7u));
-  *py = rc.sb_min[1] + (int)(by * 4u + (in >> 3));
+  *px = rc.rect_min[0] + (int)(bx * 8u + (in & 7u));
+  *py = rc.rect_min[1] + (int)(by * 4u + (in >> 3));
   *sample = rc.s_begin + (int)j * rc.s_stride;
 }
 
@@ -35,7 +35,7 @@ __global__ void __launch_bounds__(256) generate_kernel(const __grid_constant__ R
         s = list_s[i];
       } else {
         work_to_pixel(rc, work_base + i, &px, &py, &s);
-        valid = px < rc.sb_min[0] + rc.sb_ext[0] && py < rc.sb_min[1] + rc.sb_ext[1];
+        valid = px < rc.rect_min[0] + rc.rect_ext[0] && py < rc.rect_min[1] + rc.rect_ext[1];
       }
     }
     if (valid) {
@@ -70,7 +70,7 @@ __global__ void __launch_bounds__(256) generate_kernel(const __grid_constant__ R
       a.pixel = 0u;
       a.sample = 0u;
       a.spare = 0u;
-      a.fx = a.fy = -1e30f;  // padding lane of an 8x4 block outside the sample bounds
+      a.fx = a.fy = -1e30f;  // padding lane of an 8x4 block outside the enumerated rectangle
       st256(&P.slot[i].a, a);
       P.L[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }

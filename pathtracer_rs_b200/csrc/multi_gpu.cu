@@ -261,9 +261,9 @@ int32_t ptrs_multi_scene(PtrsMultiScene* multi, int32_t g, PtrsScene** scene) {
   return PTRS_OK;
 }
 
-int32_t ptrs_multi_render(PtrsMultiScene* multi, const PtrsCamera* camera, const PtrsRenderParams* params, float* host_rgbw, PtrsStats* per_device_stats,
-                          float* total_ms) {
-  if (!multi || !camera || !params) return set_error(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+int32_t ptrs_multi_render_region(PtrsMultiScene* multi, const PtrsCamera* camera, const PtrsRenderParams* params, const int32_t sample_rect[4],
+                                 float* host_rgbw, PtrsStats* per_device_stats, float* total_ms) {
+  if (!multi || !camera || !params || !sample_rect) return set_error(PTRS_ERR_INVALID_ARGUMENT, "null argument");
   const auto t0 = std::chrono::steady_clock::now();
   PtrsMultiScene& m = *multi;
   int32_t r = ensure_films(&m, camera->width, camera->height);
@@ -278,7 +278,7 @@ int32_t ptrs_multi_render(PtrsMultiScene* multi, const PtrsCamera* camera, const
     PtrsRenderParams p = *params;
     p.sample_stride = stride * m.n;
     p.sample_phase = phase + g * stride;
-    rc = ptrs_render(m.scene[g], camera, &p, m.film[g], m.stream[g]);
+    rc = ptrs_render_region(m.scene[g], camera, &p, sample_rect, m.film[g], m.stream[g]);
     if (rc != PTRS_OK) return rc;
     if (per_device_stats) rc = ptrs_stats(m.scene[g], per_device_stats + g);
     return rc;
@@ -310,6 +310,14 @@ int32_t ptrs_multi_render(PtrsMultiScene* multi, const PtrsCamera* camera, const
   }
   if (total_ms) *total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return PTRS_OK;
+}
+
+int32_t ptrs_multi_render(PtrsMultiScene* multi, const PtrsCamera* camera, const PtrsRenderParams* params, float* host_rgbw, PtrsStats* per_device_stats,
+                          float* total_ms) {
+  if (!camera || !params) return set_error(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+  int32_t bounds[4];
+  ptrs_film_sample_bounds(camera->width, camera->height, params->filter_radius, bounds);
+  return ptrs_multi_render_region(multi, camera, params, bounds, host_rgbw, per_device_stats, total_ms);
 }
 
 // ---- one process per GPU ---------------------------------------------------------------------------------

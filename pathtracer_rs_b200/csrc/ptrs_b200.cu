@@ -311,6 +311,10 @@ int32_t build_render_const(const PtrsCamera* cam, const PtrsRenderParams* rp, Re
   rc->sb_min[1] = sby0;
   rc->sb_ext[0] = sbx1 - sbx0;
   rc->sb_ext[1] = sby1 - sby0;
+  for (int k = 0; k < 2; ++k) {
+    rc->rect_min[k] = rc->sb_min[k];
+    rc->rect_ext[k] = rc->sb_ext[k];
+  }
   if (sbx0 < -32768 || sby0 < -32768 || sbx1 > 32767 || sby1 > 32767) {  // pixel coordinates travel as two int16 in the path record
     *why = "sample bounds outside the 16-bit pixel range of the path record";
     return PTRS_ERR_UNSUPPORTED;
@@ -1328,6 +1332,40 @@ int32_t ptrs_film_sample_bounds(int32_t width, int32_t height, const float r[2],
   return PTRS_OK;
 }
 
+// One axis of ptrs_film_region_sample_rect.  A sample at position s has its film coordinate fx in [s, s + 1 - 2^-24]
+// (the jitter is clamped to OneMinusEpsilon and the sum is rounded to float), and accumulate_kernel splats it onto
+// pixels ceil(fx - 0.5 - r) .. floor(fx - 0.5 + r) + 1.  Both ends grow with fx, so position s reaches a pixel of
+// [a, b) exactly when the footprint of its smallest fx starts below b and that of its largest fx ends above a.  The
+// ends are evaluated with the kernel's float expressions, not with real-number bounds.
+static void region_axis(int32_t sb0, int32_t sb1, float r, int32_t a, int32_t b, int32_t* lo, int32_t* hi) {
+  *lo = sb1;
+  *hi = sb0;
+  for (int32_t s = sb0; s < sb1; ++s) {
+    const float dx0 = (float)s - 0.5f, dx1 = ((float)s + 0x1.fffffep-1f) - 0.5f;
+    const int p0 = (int)std::ceil(dx0 - r), p1 = (int)(std::floor(dx1 + r) + 1.0f);
+    if (p0 < b && p1 > a) {
+      *lo = std::min(*lo, s);
+      *hi = std::max(*hi, s + 1);
+    }
+  }
+}
+
+int32_t ptrs_film_region_sample_rect(int32_t width, int32_t height, const float r[2], const int32_t pixel_rect[4], int32_t sample_rect[4]) {
+  if (!r || !pixel_rect || !sample_rect) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+  if (width <= 0 || height <= 0) return fail(PTRS_ERR_INVALID_ARGUMENT, "bad film resolution");
+  if (!(r[0] > 0.f) || !(r[1] > 0.f) || !(r[0] < 1024.f) || !(r[1] < 1024.f)) return fail(PTRS_ERR_INVALID_ARGUMENT, "filter radius must be positive (and finite)");
+  const int32_t size[2] = {width, height};
+  for (int k = 0; k < 2; ++k)
+    if (pixel_rect[k] < 0 || pixel_rect[k] >= pixel_rect[k + 2] || pixel_rect[k + 2] > size[k])
+      return fail(PTRS_ERR_INVALID_ARGUMENT, "pixel rectangle empty, inverted or outside the film");
+  int32_t sb[4];
+  ptrs_film_sample_bounds(width, height, r, sb);
+  int32_t out[4];
+  for (int k = 0; k < 2; ++k) region_axis(sb[k], sb[k + 2], r[k], pixel_rect[k], pixel_rect[k + 2], &out[k], &out[k + 2]);
+  std::memcpy(sample_rect, out, sizeof(out));
+  return PTRS_OK;
+}
+
 // ---- integrator ----------------------------------------------------------------------------------
 int32_t ptrs_render_params_default(PtrsRenderParams* p) {
   if (!p) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
@@ -1369,13 +1407,24 @@ static uint32_t default_paths_per_batch(PtrsScene* s) {
   return s->default_cap;
 }
 
-static int32_t render_impl(PtrsScene* s, const PtrsCamera* cam, const PtrsRenderParams* rp, PtrsFilm* film, const int32_t* list_xy,
-                           const int32_t* list_s, size_t n_list, float* out_rgb, cudaStream_t st) {
+// sample_rect: the rectangle of sample positions to trace, {x0, y0, x1, y1} half-open, inside the sample bounds
+// (ptrs_render passes the whole bounds); nullptr with a (pixel, sample number) list.
+static int32_t render_impl(PtrsScene* s, const PtrsCamera* cam, const PtrsRenderParams* rp, PtrsFilm* film, const int32_t* sample_rect,
+                           const int32_t* list_xy, const int32_t* list_s, size_t n_list, float* out_rgb, cudaStream_t st) {
   RenderConst rc;
   std::string why;
   int32_t r = build_render_const(cam, rp, &rc, &why);
   if (r != PTRS_OK) return fail(r, why);
-  const uint32_t bw = ((uint32_t)rc.sb_ext[0] + 7u) >> 3, bh = ((uint32_t)rc.sb_ext[1] + 3u) >> 2;
+  if (sample_rect) {
+    for (int k = 0; k < 2; ++k) {
+      const int32_t lo = sample_rect[k], hi = sample_rect[k + 2];
+      if (lo >= hi || lo < rc.sb_min[k] || hi > rc.sb_min[k] + rc.sb_ext[k])
+        return fail(PTRS_ERR_INVALID_ARGUMENT, "sample rectangle empty, inverted or outside the sample bounds");
+      rc.rect_min[k] = lo;
+      rc.rect_ext[k] = hi - lo;
+    }
+  }
+  const uint32_t bw = ((uint32_t)rc.rect_ext[0] + 7u) >> 3, bh = ((uint32_t)rc.rect_ext[1] + 3u) >> 2;
   const uint64_t per_sample = (uint64_t)bw * bh * 32u;
   const uint64_t total = list_xy ? (uint64_t)n_list : per_sample * (uint64_t)rc.s_count;
   // Wavefront batch size.  Every batch pays for its tail: the rounds after Russian roulette has thinned the paths out are
@@ -1438,8 +1487,8 @@ static int32_t render_impl(PtrsScene* s, const PtrsCamera* cam, const PtrsRender
   tm.collect(ms);
   float total_ms = 0.f;
   cudaEventElapsedTime(&total_ms, s->ev[0], s->ev[1]);
-  // camera paths = valid (pixel, sample) pairs; 8x4 block padding outside the sample bounds is not counted
-  paths = list_xy ? n_list : (uint64_t)rc.sb_ext[0] * rc.sb_ext[1] * (uint64_t)rc.s_count;
+  // camera paths = valid (pixel, sample) pairs; 8x4 block padding outside the enumerated rectangle is not counted
+  paths = list_xy ? n_list : (uint64_t)rc.rect_ext[0] * rc.rect_ext[1] * (uint64_t)rc.s_count;
   s->stats.camera_paths = paths;
   s->stats.extension_rays = ext_rays;
   s->stats.shadow_rays = g.shadow_rays;
@@ -1459,14 +1508,22 @@ static int32_t render_impl(PtrsScene* s, const PtrsCamera* cam, const PtrsRender
   return PTRS_OK;
 }
 
-int32_t ptrs_render(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params, PtrsFilm* film, void* stream) {
-  if (!scene || !camera || !params || !film) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+int32_t ptrs_render_region(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params, const int32_t sample_rect[4], PtrsFilm* film,
+                           void* stream) {
+  if (!scene || !camera || !params || !sample_rect || !film) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
   if (film->width != camera->width || film->height != camera->height) return fail(PTRS_ERR_INVALID_ARGUMENT, "film / camera resolution mismatch");
   if (film->device != scene->device) return fail(PTRS_ERR_INVALID_ARGUMENT, "film and scene live on different devices");
   ON_DEVICE_OF(scene);
-  const int32_t r = render_impl(scene, camera, params, film, nullptr, nullptr, 0, nullptr, (cudaStream_t)stream);
+  const int32_t r = render_impl(scene, camera, params, film, sample_rect, nullptr, nullptr, 0, nullptr, (cudaStream_t)stream);
   if (r != PTRS_OK) cudaStreamSynchronize((cudaStream_t)stream);  // nothing of the failed call may still run when its buffers are released
   return r;
+}
+
+int32_t ptrs_render(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params, PtrsFilm* film, void* stream) {
+  if (!camera || !params) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
+  int32_t bounds[4];
+  ptrs_film_sample_bounds(camera->width, camera->height, params->filter_radius, bounds);
+  return ptrs_render_region(scene, camera, params, bounds, film, stream);
 }
 
 int32_t ptrs_path_radiance(PtrsScene* scene, const PtrsCamera* camera, const PtrsRenderParams* params, const int32_t* pixels_xy,
@@ -1474,7 +1531,7 @@ int32_t ptrs_path_radiance(PtrsScene* scene, const PtrsCamera* camera, const Ptr
   if (!scene || !camera || !params || (n && (!pixels_xy || !sample_nums || !out_rgb))) return fail(PTRS_ERR_INVALID_ARGUMENT, "null argument");
   if (n == 0) return PTRS_OK;
   ON_DEVICE_OF(scene);
-  const int32_t r = render_impl(scene, camera, params, nullptr, pixels_xy, sample_nums, n, out_rgb, 0);
+  const int32_t r = render_impl(scene, camera, params, nullptr, nullptr, pixels_xy, sample_nums, n, out_rgb, 0);
   if (r != PTRS_OK) cudaStreamSynchronize(0);
   return r;
 }

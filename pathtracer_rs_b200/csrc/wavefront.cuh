@@ -157,6 +157,9 @@ struct RenderConst {
   int32_t rr_start_depth;
   int32_t rr_enable;
   int32_t sb_min[2], sb_ext[2];  // sample bounds min and extent
+  // the rectangle of sample positions the generate kernel enumerates: the sample bounds or a sub-rectangle of them
+  // (ptrs_render_region).  The Sobol index and the split tables stay relative to the full sample bounds.
+  int32_t rect_min[2], rect_ext[2];
   int32_t s_begin, s_count, s_stride, s_phase;  // sample numbers: s = s_begin + s_phase' + j * s_stride
   uint32_t cap;
 };

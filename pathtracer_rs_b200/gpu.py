@@ -33,7 +33,7 @@ EXPORTS = [
     "ptrs_multi_create", "ptrs_multi_destroy", "ptrs_multi_device_count", "ptrs_multi_render", "ptrs_multi_root_film", "ptrs_multi_scene",
     "ptrs_comm_unique_id", "ptrs_comm_init_rank", "ptrs_comm_destroy", "ptrs_comm_info", "ptrs_film_reduce",
     "ptrs_bxdf_eval", "ptrs_bxdf_sample", "ptrs_light_sample", "ptrs_light_pdf", "ptrs_scene_download_mipmaps", "ptrs_scene_download_env",
-    "ptrs_scene_create_sah_bvh",
+    "ptrs_scene_create_sah_bvh", "ptrs_render_region", "ptrs_multi_render_region", "ptrs_film_region_sample_rect",
 ]
 
 
@@ -83,8 +83,10 @@ def lib():
         L.ptrs_film_device_ptr.restype = vp
         L.ptrs_film_device_ptr.argtypes = [vp]
         L.ptrs_film_sample_bounds.argtypes = [i32, i32, fp, i32p]
+        L.ptrs_film_region_sample_rect.argtypes = [i32, i32, fp, i32p, i32p]
         L.ptrs_render_params_default.argtypes = [rpp]
         L.ptrs_render.argtypes = [vp, camp, rpp, vp, vp]
+        L.ptrs_render_region.argtypes = [vp, camp, rpp, i32p, vp, vp]
         L.ptrs_path_radiance.argtypes = [vp, camp, rpp, i32p, i32p, sz, fp]
         L.ptrs_stats.argtypes = [vp, C.POINTER(PtrsStats)]
         L.ptrs_set_stats_mode.argtypes = [vp, i32]
@@ -96,6 +98,7 @@ def lib():
         L.ptrs_multi_destroy.argtypes = [vp]
         L.ptrs_multi_device_count.argtypes = [vp, i32p]
         L.ptrs_multi_render.argtypes = [vp, camp, rpp, fp, C.POINTER(PtrsStats), fp]
+        L.ptrs_multi_render_region.argtypes = [vp, camp, rpp, i32p, fp, C.POINTER(PtrsStats), fp]
         L.ptrs_multi_root_film.argtypes = [vp, C.POINTER(vp)]
         L.ptrs_multi_scene.argtypes = [vp, i32, C.POINTER(vp)]
         L.ptrs_comm_unique_id.argtypes = [u8p]
@@ -119,6 +122,13 @@ def _check(rc):
 
 def _p(a, t):
     return a.ctypes.data_as(C.POINTER(t))
+
+
+def _rect(r):
+    """(x0, y0, x1, y1) -> int32_t[4]"""
+    if len(r) != 4:
+        raise ValueError("a rectangle is (x0, y0, x1, y1)")
+    return (C.c_int32 * 4)(*(int(v) for v in r))
 
 
 def device_count():
@@ -175,6 +185,14 @@ class Film:
         r = (C.c_float * 2)(*radius)
         out = (C.c_int32 * 4)()
         _check(lib().ptrs_film_sample_bounds(self.width, self.height, r, out))
+        return tuple(out)
+
+    def region_sample_rect(self, pixel_rect, radius=(2.0, 2.0)):
+        """The sample rectangle whose render completes the pixels of pixel_rect (x0, y0, x1, y1), half-open
+        (ptrs_film_region_sample_rect); pass it to PathIntegrator.render(..., region=...)."""
+        r = (C.c_float * 2)(*radius)
+        out = (C.c_int32 * 4)()
+        _check(lib().ptrs_film_region_sample_rect(self.width, self.height, r, _rect(pixel_rect), out))
         return tuple(out)
 
     def download(self):
@@ -367,12 +385,18 @@ class MultiScene:
         _check(lib().ptrs_multi_create(desc, n_devices, dv, 1 if device_bvh else 0, C.byref(h)))
         self._h, self.n_devices = h, n_devices
 
-    def render(self, camera, params, download=True):
-        """PathIntegrator::render over all devices.  Returns (raw film sums (H, W, 4) or None, per-device stats, total ms)."""
+    def render(self, camera, params, download=True, region=None):
+        """PathIntegrator::render over all devices.  Returns (raw film sums (H, W, 4) or None, per-device stats, total ms).
+        region: a rectangle of sample positions (x0, y0, x1, y1) to trace instead of the whole sample bounds
+        (ptrs_multi_render_region); the film is still reduced and downloaded whole."""
         out = np.empty((camera.height, camera.width, 4), dtype=np.float32) if download else None
         st = (PtrsStats * self.n_devices)()
         ms = C.c_float(0)
-        _check(lib().ptrs_multi_render(self._h, C.byref(camera), C.byref(params), _p(out, C.c_float) if download else None, st, C.byref(ms)))
+        host = _p(out, C.c_float) if download else None
+        if region is None:
+            _check(lib().ptrs_multi_render(self._h, C.byref(camera), C.byref(params), host, st, C.byref(ms)))
+        else:
+            _check(lib().ptrs_multi_render_region(self._h, C.byref(camera), C.byref(params), _rect(region), host, st, C.byref(ms)))
         stats = [{k: getattr(s, k) for k, _ in PtrsStats._fields_} for s in st]
         return out, stats, ms.value
 
@@ -420,17 +444,21 @@ class PathIntegrator:
     def preprocess(self, scene):  # integrator.rs:250-258
         self.too_many_lights = scene.n_lights > 16
 
-    def render(self, camera, scene, film, stream=None, sample_range=None, sample_stride=(1, 0), exact_shading=False):
+    def render(self, camera, scene, film, stream=None, sample_range=None, sample_stride=(1, 0), exact_shading=False, region=None):
         """integrator.rs:536 — accumulates into `film` (the reference's camera.film).  sample_range /
         sample_stride select a shard of the Sobol sample numbers (multi-GPU); exact_shading selects the parity
-        build of the shade kernels (PTRS_RENDER_EXACT_SHADING)."""
+        build of the shade kernels (PTRS_RENDER_EXACT_SHADING); region (x0, y0, x1, y1) traces only that rectangle of
+        sample positions (ptrs_render_region; Film.region_sample_rect gives the one that completes a pixel crop)."""
         p = PtrsRenderParams.from_buffer_copy(self.params)
         if exact_shading:
             p.flags |= RENDER_EXACT_SHADING
         if sample_range is not None:
             p.sample_begin, p.sample_end = sample_range
         p.sample_stride, p.sample_phase = sample_stride
-        _check(lib().ptrs_render(scene._h, C.byref(camera), C.byref(p), film._h, C.c_void_p(stream or 0)))
+        if region is None:
+            _check(lib().ptrs_render(scene._h, C.byref(camera), C.byref(p), film._h, C.c_void_p(stream or 0)))
+        else:
+            _check(lib().ptrs_render_region(scene._h, C.byref(camera), C.byref(p), _rect(region), film._h, C.c_void_p(stream or 0)))
         return scene.stats()
 
 

@@ -47,6 +47,13 @@ class Film {
     check(ptrs_film_sample_bounds(w_, h_, radius, b));
     return Bounds2i{b[0], b[1], b[2], b[3]};
   }
+  // the sample rectangle whose render completes the pixels of pixel_rect (ptrs_film_region_sample_rect)
+  Bounds2i region_sample_rect(const Bounds2i& pixel_rect, const float radius[2]) const {
+    const int32_t p[4] = {pixel_rect.x0, pixel_rect.y0, pixel_rect.x1, pixel_rect.y1};
+    int32_t b[4];
+    check(ptrs_film_region_sample_rect(w_, h_, radius, p, b));
+    return Bounds2i{b[0], b[1], b[2], b[3]};
+  }
   std::vector<uint8_t> to_rgba_image() const {                                           // film.rs:230-251
     std::vector<uint8_t> out((size_t)w_ * h_ * 4);
     check(ptrs_film_resolve_srgb8(f_, out.data()));
@@ -137,6 +144,11 @@ class PathIntegrator {
   void toggle_progress_bar() { progress_ = !progress_; }
   void render(Camera& camera, const RenderScene& scene) const {  // integrator.rs:536: accumulates into camera.film
     check(ptrs_render(scene.handle(), &camera.cam, &params_, camera.film.handle(), nullptr));
+  }
+  // the same restricted to a rectangle of sample positions (ptrs_render_region), e.g. one tile of integrator.rs:545-637
+  void render(Camera& camera, const RenderScene& scene, const Bounds2i& sample_rect) const {
+    const int32_t r[4] = {sample_rect.x0, sample_rect.y0, sample_rect.x1, sample_rect.y1};
+    check(ptrs_render_region(scene.handle(), &camera.cam, &params_, r, camera.film.handle(), nullptr));
   }
   PtrsStats stats(const RenderScene& scene) const {
     PtrsStats st;
